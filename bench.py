@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: grid-points/s, forward+backward, Darcy 141^2 Galerkin-transformer (BASELINE C3).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload ("darcy141_galerkin10_sc2d_b8"): FourierTransformer2D with the reference's ex2_darcy
 configuration (config.yml:41-80) at the reference's own profiling protocol
@@ -20,6 +20,9 @@ Lines printed (rank 0): one JSON object, see the keys in `main`.
   cpu_baseline : the oracle (CPU restatement of the reference) timed on this box's host cores
 --impl reference : the oracle on CPU only, same metric/config (the reference is pure PyTorch and
   cannot travel to the GPU box; the oracle is pinned to it by tests/golden).
+--dump-outputs DIR : after the timed steps, what the last timed step handed its caller -- the loss and the gradient of
+  every parameter -- as DIR/loss.npy and DIR/grad.<parameter name>.npy (float32, rank 0).  Inputs, weights and dropout
+  streams are seeded, so two builds run with the same arguments can be compared array for array.
 """
 import argparse
 import json
@@ -327,6 +330,22 @@ def ncu_traffic(kernel):
     return None
 
 
+DUMP_LIMIT_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(out_dir, loss, model):
+    """Write the loss and every parameter gradient of the last timed step as float32 .npy files; returns the file count."""
+    import numpy as np
+    arrays = {"loss": loss}
+    arrays.update((f"grad.{n}", p.grad) for n, p in model.named_parameters() if p.grad is not None)
+    total = sum(t.numel() * 4 for t in arrays.values())
+    assert total <= DUMP_LIMIT_BYTES, f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit"
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+    return len(arrays)
+
+
 def kernel_table(summary, steps, peaks):
     """Per kernel family: launches/step, ms/step, achieved GB/s and TFLOP/s on ALGORITHMIC work."""
     rows = []
@@ -369,7 +388,13 @@ def main():
     ap.add_argument("--precision", default="x3", choices=["x3", "tf32", "fp32"],
                     help="x3 (default): bf16x3 fused encoder / conv kernels + TF32 weight gradients + exact fp32 elsewhere; "
                          "tf32: every GEMM single-pass TF32; fp32: exact SIMT")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's loss and parameter gradients to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the b200 implementation only")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -477,7 +502,7 @@ def main():
     for i in range(args.steps):
         flush.fill_(float(i))
         starts[i].record()
-        step(*resident)
+        last_loss = step(*resident)
         ends[i].record()
     barrier()
     wall = time.perf_counter() - wall0
@@ -492,6 +517,9 @@ def main():
     total_ms = t.item()
     ms_per_step = total_ms / args.steps
     value = bsz * world * wl.points / (ms_per_step * 1e-3)
+    if args.dump_outputs and rank == 0:       # before the passes below overwrite the gradients
+        n = dump_outputs(args.dump_outputs, last_loss, model)
+        log(f"wrote {n} arrays of the last timed step to {args.dump_outputs}")
 
     log(f"device-timed: {ms_per_step:.3f} ms/step; end-to-end pass")
     # ---- end to end: pinned host inputs -> H2D -> fwd+bwd -> D2H loss, every step ------------

@@ -14,25 +14,20 @@ With this repository on PYTHONPATH the reference's `examples/*.py` run unchanged
   * ``galerkin_transformer.utils / utils_ft / ft`` = the reference's own files (datasets, losses, training loop: out of
     scope here, SURVEY.md section 8).
 
-The reference sources are looked up in $GALERKIN_REFERENCE, `<repo>/baseline/_ref` (git-ignored staging copy made by
-`tools/stage_reference.py`; it travels to the GPU box) or `/root/reference`.  Without them only the B200 classes are
-exported.  `torchinfo`, `matplotlib` and `IPython` are optional for the reference's utilities; minimal stand-ins are
-registered when they are not installed."""
+The reference sources are looked up in $GALERKIN_REFERENCE (the root of a checkout of the reference).  Without them
+only the B200 classes are exported.  `torchinfo`, `matplotlib` and `IPython` are optional for the reference's
+utilities; minimal stand-ins are registered when they are not installed."""
 import importlib.util
 import os
 import sys
 import types
 
-_HERE = os.path.dirname(os.path.abspath(__file__))
-_REPO = os.path.dirname(_HERE)
-
 
 def reference_libs():
     """directory holding the reference's layers.py / model.py / ..., or None"""
-    cands = [os.environ.get("GALERKIN_REFERENCE"), os.path.join(_REPO, "baseline", "_ref"), "/root/reference"]
-    for root in cands:
-        if root and os.path.isfile(os.path.join(root, "libs", "layers.py")):
-            return os.path.join(root, "libs")
+    root = os.environ.get("GALERKIN_REFERENCE")
+    if root and os.path.isfile(os.path.join(root, "libs", "layers.py")):
+        return os.path.join(root, "libs")
     return None
 
 

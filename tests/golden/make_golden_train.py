@@ -1,11 +1,11 @@
 """Fixtures that pin oracle/train_oracle.py (and, on the GPU box, csrc/train.cu) to the reference's own loss class.
 
-Runs ONLY in the build container (needs /root/reference): imports libs/ft.py's WeightedL2Loss2d through the
+Needs a checkout of the reference: imports libs/ft.py's WeightedL2Loss2d through the
 `galerkin_transformer` alias package (which stubs the plotting imports), evaluates it on seeded inputs the way
 train_batch_darcy does (libs/utils_ft.py:672-674: loss_func(u_pred, u, targets_prime=gradu, K=a)), and records the
 outputs and the autograd gradients of the loss and of the regulariser w.r.t. preds in tests/golden/train/<case>.pt.
 
-    python tests/golden/make_golden_train.py"""
+    GALERKIN_REFERENCE=/path/to/reference python tests/golden/make_golden_train.py"""
 import os
 import sys
 
@@ -23,6 +23,7 @@ CASES = [dict(name="loss_h1_k", B=3, n=17, regularizer=True, gamma=0.5, use_K=Tr
 
 def main():
     ft = load_reference_module("ft")
+    assert ft is not None, "set GALERKIN_REFERENCE to the root of a checkout of the reference"
     os.makedirs(os.path.join(HERE, "train"), exist_ok=True)
     for i, c in enumerate(CASES):
         g = torch.Generator().manual_seed(4100 + i)

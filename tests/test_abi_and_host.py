@@ -7,6 +7,7 @@ import glob
 import os
 import pickle
 import re
+import types
 
 import pytest
 import torch
@@ -71,6 +72,32 @@ def test_state_dict_layout_matches_reference(name):
     clone = copy.deepcopy(mod)                     # model.py:896, 1153 deepcopy the layer
     blob = pickle.dumps(mod)                       # utils_ft.py:804 pickles whole models
     assert list(pickle.loads(blob).state_dict().keys()) == list(clone.state_dict().keys())
+
+
+def test_dropin_patch_rebinds_module_namespaces():
+    """dropin.patch rebinds the hot-path classes in stand-ins for the reference's `layers` / `model` modules, whose
+    assembly code looks its classes up in the module namespace at call time; assembly classes stay untouched."""
+    from galerkin_transformer_b200.dropin import LAYER_CLASSES, MODEL_CLASSES, patch
+    layers, model = types.ModuleType("layers"), types.ModuleType("model")
+    for n in LAYER_CLASSES:
+        setattr(layers, n, type(n, (torch.nn.Module,), {}))
+    for n in MODEL_CLASSES + ("FourierTransformer2D",):
+        setattr(model, n, type(n, (torch.nn.Module,), {}))
+    model.SimpleAttention = layers.SimpleAttention          # what `from layers import *` leaves in libs/model.py
+    assembly = model.FourierTransformer2D
+    exec("def encoder_layer(**kw):\n    return SimpleTransformerEncoderLayer(**kw)\n", vars(model))
+
+    done = patch(layers, model)
+    assert done == {"layers": list(LAYER_CLASSES), "model": ["SimpleAttention", *MODEL_CLASSES]}
+    for ns, names in ((layers, LAYER_CLASSES), (model, MODEL_CLASSES + ("SimpleAttention",))):
+        for n in names:
+            assert getattr(ns, n) is getattr(G, n), n
+    assert model.FourierTransformer2D is assembly
+    fix = load_golden("enc_galerkin_attnnorm")
+    layer = model.encoder_layer(**fix["config"])
+    assert isinstance(layer, G.SimpleTransformerEncoderLayer) and isinstance(layer.attn, G.SimpleAttention)
+    assert list(layer.state_dict().keys()) == list(fix["state_dict"].keys())
+    layer.load_state_dict(fix["state_dict"])
 
 
 def test_no_cpu_fallback():

@@ -59,19 +59,16 @@ SIGNATURES = {
                            c_vp, c_int, c_float, c_int, c_int, c_vp, c_sz, c_vp]),
     "gb200_gemm_tc_supported": (c_int, [c_vp, c_int, c_vp, c_int, c_int, c_int, c_int]),
     "gb200_gemm_tc_suggest_ksplit": (c_int, [c_int] * 3),
-    "gb200_gemm_tc_split_next": (c_int, [c_int]),
     "gb200_gemm_tc_wgrad_group_workspace_bytes": (c_sz, [c_int, ctypes.POINTER(WgradProblem)]),
     "gb200_gemm_tc_wgrad_group": (c_int, [c_int, c_int, ctypes.POINTER(WgradProblem), c_vp, c_sz, c_vp]),
     "gb200_gemm_tc_set_trace": (c_int, [c_vp]),
     "gb200_gemm_tc": (c_int, [c_int, c_vp, c_int, c_int, c_vp, c_int, c_int, c_vp, c_int, c_int, c_int, c_int,
                               c_float, c_vp, c_int, c_vp, c_int, c_float, c_ull, c_vp, c_int, c_float, c_int,
-                              c_int, c_vp, c_sz, c_vp]),
+                              c_int, c_vp, c_sz, c_int, c_vp]),
     "gb200_gemm_tc_gated": (c_int, [c_int, c_vp, c_int, c_int, c_vp, c_int, c_int, c_vp, c_int, c_int, c_int, c_int, c_float, c_float,
-                                    c_ull, c_float, c_vp, c_int, c_int, c_int, c_vp, c_sz, c_vp]),
+                                    c_ull, c_float, c_vp, c_int, c_int, c_int, c_vp, c_sz, c_int, c_vp]),
     "gb200_gemm_gated": (c_int, [c_int, c_vp, c_int, c_int, c_vp, c_int, c_int, c_vp, c_int, c_int, c_int, c_int, c_float, c_float,
                                     c_ull, c_float, c_vp, c_int, c_int, c_int, c_vp, c_sz, c_vp]),
-    "gb200_gemm_tc_headnorm": (c_int, [c_int, c_vp, c_int, c_vp, c_int, c_vp, c_int, c_int, c_int, c_int, c_vp, c_int,
-                                       c_int, c_int, c_int, c_float, c_vp, c_vp, c_vp]),
     "gb200_colsum_workspace_bytes": (c_sz, [c_ll, c_int]),
     "gb200_colsum": (c_int, [c_int, c_vp, c_int, c_ll, c_int, c_float, c_int, c_vp, c_vp, c_sz, c_vp]),
     "gb200_epilogue_bwd": (c_int, [c_int, c_vp, c_int, c_vp, c_int, c_vp, c_int, c_vp, c_int, c_ll, c_int,

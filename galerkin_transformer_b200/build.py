@@ -34,7 +34,7 @@ def build(force=False, verbose=False):
     if not force and not is_stale():
         return OUT
     nvcc = os.environ.get("NVCC", "nvcc")
-    extra = os.environ.get("GB200_NVCC_EXTRA", "").split()      # tuning experiments: e.g. -DGB200_PDL_MODE=0
+    extra = os.environ.get("GB200_NVCC_EXTRA", "").split()      # extra nvcc flags for experiments: e.g. -Xptxas -warn-spills
     os.makedirs(OBJ_DIR, exist_ok=True)
     tag = os.path.join(OBJ_DIR, ".flags")
     flags_now = " ".join(NVCC_FLAGS + extra)

@@ -14,7 +14,6 @@
 //   libs/layers.py:723, 728, 733      K^T V, /n, Q.(.)           (linear_attention)
 //   libs/layers.py:730-731            F.dropout(p_attn), p=0.5, always on (mask input)
 //   libs/layers.py:892-894            transpose(1,2).contiguous().view  (head merge)
-#include <stdlib.h>
 #include "common.cuh"
 #include "head_operand.cuh"
 #include "attention_mma.cuh"
@@ -404,7 +403,7 @@ extern "C" int gb200_headnorm_fwd(int device, float* x, int ld, int col0, int co
         int blocks = cdiv(T, rpb);
         if (blocks > HN_VEC_BLOCKS) blocks = HN_VEC_BLOCKS;
         dim3 grid(blocks, nblk);
-#define HN_FWD(LG) launch_pdl(headnorm_fwd_vec_kernel<LG>, grid, 256, 0, st, x, ld, blk, T, H, dk, eps)
+#define HN_FWD(LG) launch_kernel(headnorm_fwd_vec_kernel<LG>, grid, 256, 0, st, x, ld, blk, T, H, dk, eps)
         switch (lg) { case 1: HN_FWD(1); break; case 2: HN_FWD(2); break; case 4: HN_FWD(4); break;
                       case 8: HN_FWD(8); break; case 16: HN_FWD(16); break; default: HN_FWD(32); }
 #undef HN_FWD
@@ -414,8 +413,8 @@ extern "C" int gb200_headnorm_fwd(int device, float* x, int ld, int col0, int co
     GB_REQUIRE(smem <= 200 * 1024, "gb200_headnorm_fwd: H*d_k=%d too wide", H * dk);
     if (smem > 48 * 1024)
         cudaFuncSetAttribute(headnorm_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    launch_pdl(headnorm_fwd_kernel, cdiv(T, HN_ROWS), 256, smem, st, x, ld, col0, T, H, dk, eps, rstd);
-    if (nblk == 2) launch_pdl(headnorm_fwd_kernel, cdiv(T, HN_ROWS), 256, smem, st, x, ld, col0b, T, H, dk, eps, rstd_b);
+    launch_kernel(headnorm_fwd_kernel, cdiv(T, HN_ROWS), 256, smem, st, x, ld, col0, T, H, dk, eps, rstd);
+    if (nblk == 2) launch_kernel(headnorm_fwd_kernel, cdiv(T, HN_ROWS), 256, smem, st, x, ld, col0b, T, H, dk, eps, rstd_b);
     return check_launch("gb200_headnorm_fwd", nblk);
 }
 
@@ -456,14 +455,14 @@ extern "C" int gb200_headnorm_bwd(int device, float* dy, int lddy, int dcol0, in
         blk.rstd[0] = const_cast<float*>(rstd); blk.rstd[1] = const_cast<float*>(rstd_b);
         blk.gamma[0] = gamma; blk.gamma[1] = gamma_b; blk.part[0] = part_a; blk.part[1] = part_b;
         dim3 grid(blocks, nblk);
-#define HN_BWD(LG) launch_pdl(headnorm_bwd_vec_kernel<LG>, grid, 256, 0, st, dy, lddy, xhat, ldx, blk, T, H, dk)
+#define HN_BWD(LG) launch_kernel(headnorm_bwd_vec_kernel<LG>, grid, 256, 0, st, dy, lddy, xhat, ldx, blk, T, H, dk)
         switch (lg) { case 1: HN_BWD(1); break; case 2: HN_BWD(2); break; case 4: HN_BWD(4); break;
                       case 8: HN_BWD(8); break; case 16: HN_BWD(16); break; default: HN_BWD(32); }
 #undef HN_BWD
-        launch_pdl(headnorm_bwd_reduce_kernel, dim3(cdiv(W, 32), 2), dim3(32, 32), 0, st, part_a, blocks, W, dgamma, dbeta,
+        launch_kernel(headnorm_bwd_reduce_kernel, dim3(cdiv(W, 32), 2), dim3(32, 32), 0, st, part_a, blocks, W, dgamma, dbeta,
                                                                                 accumulate);
         if (nblk == 2)
-            launch_pdl(headnorm_bwd_reduce_kernel, dim3(cdiv(W, 32), 2), dim3(32, 32), 0, st, part_b, blocks, W, dgamma_b,
+            launch_kernel(headnorm_bwd_reduce_kernel, dim3(cdiv(W, 32), 2), dim3(32, 32), 0, st, part_b, blocks, W, dgamma_b,
                                                                                     dbeta_b, accumulate);
         return check_launch("gb200_headnorm_bwd", 1 + nblk);
     }
@@ -473,13 +472,13 @@ extern "C" int gb200_headnorm_bwd(int device, float* dy, int lddy, int dcol0, in
         cudaFuncSetAttribute(headnorm_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     const int nblocks = cdiv(T, HN_ROWS);
     float* part_b = workspace + (size_t)nblocks * 2 * W;
-    launch_pdl(headnorm_bwd_kernel, nblocks, 256, smem, st, dy, lddy, dcol0, xhat, ldx, xcol0, rstd, gamma, T, H, dk, part_a);
-    launch_pdl(headnorm_bwd_reduce_kernel, dim3(cdiv(W, 32), 2), dim3(32, 32), 0, st, part_a, nblocks, W, dgamma, dbeta,
+    launch_kernel(headnorm_bwd_kernel, nblocks, 256, smem, st, dy, lddy, dcol0, xhat, ldx, xcol0, rstd, gamma, T, H, dk, part_a);
+    launch_kernel(headnorm_bwd_reduce_kernel, dim3(cdiv(W, 32), 2), dim3(32, 32), 0, st, part_a, nblocks, W, dgamma, dbeta,
                                                                             accumulate);
     if (nblk == 2) {
-        launch_pdl(headnorm_bwd_kernel, nblocks, 256, smem, st, dy, lddy, dcol0b, xhat, ldx, xcol0b, rstd_b, gamma_b, T, H, dk,
+        launch_kernel(headnorm_bwd_kernel, nblocks, 256, smem, st, dy, lddy, dcol0b, xhat, ldx, xcol0b, rstd_b, gamma_b, T, H, dk,
                                                         part_b);
-        launch_pdl(headnorm_bwd_reduce_kernel, dim3(cdiv(W, 32), 2), dim3(32, 32), 0, st, part_b, nblocks, W, dgamma_b,
+        launch_kernel(headnorm_bwd_reduce_kernel, dim3(cdiv(W, 32), 2), dim3(32, 32), 0, st, part_b, nblocks, W, dgamma_b,
                                                                                 dbeta_b, accumulate);
     }
     return check_launch("gb200_headnorm_bwd", 2 * nblk);
@@ -487,9 +486,8 @@ extern "C" int gb200_headnorm_bwd(int device, float* dy, int lddy, int dcol0, in
 
 extern "C" int gb200_attn_suggest_nsplit(int B, int H, int n) {
     // The kernel is latency-bound (stage tokens -> sync -> contract): give every 64-token stage its own CTA so all
-    // loads of the launch are in flight at once, instead of a few CTAs looping over stages.  Tunable for A/B runs.
-    static const int per = []() { const char* v = getenv("GB200_XTY_TOKENS_PER_CTA"); return v ? atoi(v) : 64; }();
-    int s = (n + per - 1) / per;
+    // loads of the launch are in flight at once, instead of a few CTAs looping over stages.
+    int s = (n + 63) / 64;
     if (s > 64) s = 64;
     return s < 1 ? 1 : s;
 }
@@ -518,19 +516,19 @@ extern "C" int gb200_attn_xty(int device, const gb200_head_operand* L, const gb2
     cudaStream_t st = as_stream(stream);
     HeadOperand l = make_op(L), r = make_op(R);
     if (tensor_cores && d <= 64) {       // warp-level TF32 MMA, tiles right-sized to d
-        if (d <= 24) launch_pdl(xty_mma_kernel<2, 3>, grid, 256, 0, st, l, r, pos, p, dk, H, n, nsplit, chunk, workspace);
-        else if (d <= 40) launch_pdl(xty_mma_kernel<3, 5>, grid, 256, 0, st, l, r, pos, p, dk, H, n, nsplit, chunk, workspace);
-        else if (d <= 56) launch_pdl(xty_mma_kernel<4, 7>, grid, 256, 0, st, l, r, pos, p, dk, H, n, nsplit, chunk, workspace);
-        else launch_pdl(xty_mma_kernel<4, 8>, grid, 256, 0, st, l, r, pos, p, dk, H, n, nsplit, chunk, workspace);
+        if (d <= 24) launch_kernel(xty_mma_kernel<2, 3>, grid, 256, 0, st, l, r, pos, p, dk, H, n, nsplit, chunk, workspace);
+        else if (d <= 40) launch_kernel(xty_mma_kernel<3, 5>, grid, 256, 0, st, l, r, pos, p, dk, H, n, nsplit, chunk, workspace);
+        else if (d <= 56) launch_kernel(xty_mma_kernel<4, 7>, grid, 256, 0, st, l, r, pos, p, dk, H, n, nsplit, chunk, workspace);
+        else launch_kernel(xty_mma_kernel<4, 8>, grid, 256, 0, st, l, r, pos, p, dk, H, n, nsplit, chunk, workspace);
     } else
-    if (dp == 32) launch_pdl(xty_kernel<32>, grid, 256, 0, st, l, r, pos, p, dk, H, n, nsplit, chunk, workspace);
-    else if (dp == 64) launch_pdl(xty_kernel<64>, grid, 256, 0, st, l, r, pos, p, dk, H, n, nsplit, chunk, workspace);
-    else launch_pdl(xty_kernel<128>, grid, 256, 0, st, l, r, pos, p, dk, H, n, nsplit, chunk, workspace);
+    if (dp == 32) launch_kernel(xty_kernel<32>, grid, 256, 0, st, l, r, pos, p, dk, H, n, nsplit, chunk, workspace);
+    else if (dp == 64) launch_kernel(xty_kernel<64>, grid, 256, 0, st, l, r, pos, p, dk, H, n, nsplit, chunk, workspace);
+    else launch_kernel(xty_kernel<128>, grid, 256, 0, st, l, r, pos, p, dk, H, n, nsplit, chunk, workspace);
     long long total = (long long)B * H * d * d;
     int blocks = (int)((total + 255) / 256);
     if (blocks > 148 * 8) blocks = 148 * 8;
     GB_REQUIRE(mask_p >= 0.f && mask_p < 1.f, "gb200_attn_xty: mask_p=%f outside [0,1)", mask_p);
-    launch_pdl(xty_reduce_kernel, blocks, 256, 0, st, workspace, nsplit, d * d, total, scale, keep_mask, mask_p, mask_seed,
+    launch_kernel(xty_reduce_kernel, blocks, 256, 0, st, workspace, nsplit, d * d, total, scale, keep_mask, mask_p, mask_seed,
                                               rng_offset_ptr(), out);
     return check_launch("gb200_attn_xty", 2);
 }
@@ -552,7 +550,7 @@ extern "C" int gb200_philox_scale(int device, float* out, long long total, float
     if (total == 0) return GB200_OK;
     int blocks = (int)((total + 255) / 256);
     if (blocks > 148 * 8) blocks = 148 * 8;
-    launch_pdl(philox_scale_kernel, blocks, 256, 0, as_stream(stream), out, total, p, seed, rng_offset_ptr());
+    launch_kernel(philox_scale_kernel, blocks, 256, 0, as_stream(stream), out, total, p, seed, rng_offset_ptr());
     return check_launch("gb200_philox_scale");
 }
 
@@ -571,7 +569,7 @@ extern "C" int gb200_attn_xm(int device, const gb200_head_operand* L, const floa
     HeadOperand l = make_op(L);
     if (tensor_cores && d <= 64) {
 #define LAUNCH_XMM(KT, NT, TT)                                                                               \
-    launch_pdl(xm_mma_kernel<KT, NT, TT>, dim3(cdiv(n, TT), B * H), TT * 2, 0, st, l, pos, M, transM, p, dk, H, n, out, ldo, \
+    launch_kernel(xm_mma_kernel<KT, NT, TT>, dim3(cdiv(n, TT), B * H), TT * 2, 0, st, l, pos, M, transM, p, dk, H, n, out, ldo, \
                                                                            ocol0, out_augmented, out_scale)
         if (d <= 24) LAUNCH_XMM(3, 3, 128);
         else if (d <= 40) LAUNCH_XMM(5, 5, 128);
@@ -584,7 +582,7 @@ extern "C" int gb200_attn_xm(int device, const gb200_head_operand* L, const floa
     do {                                                                                                \
         if (smem > 48 * 1024)                                                                           \
             cudaFuncSetAttribute(xm_kernel<DPV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-        launch_pdl(xm_kernel<DPV>, grid, 256, smem, st, l, pos, M, transM, p, dk, H, n, out, ldo, ocol0,          \
+        launch_kernel(xm_kernel<DPV>, grid, 256, smem, st, l, pos, M, transM, p, dk, H, n, out, ldo, ocol0,          \
                                                out_augmented, out_scale);                               \
     } while (0)
     if (dp == 32) LAUNCH_XM(32);

@@ -221,7 +221,7 @@ template <typename K>
 static void launch_quad(K kernel, const QuadArgs& a, size_t smem, cudaStream_t st) {
     if (smem > 48 * 1024) cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     dim3 grid(cdiv(a.n, QT), a.B * a.H);
-    launch_pdl(kernel, grid, 256, smem, st, a);
+    launch_kernel(kernel, grid, 256, smem, st, a);
 }
 
 extern "C" int gb200_fourier_quad_fwd(int device, const gb200_head_operand* q, const gb200_head_operand* k,

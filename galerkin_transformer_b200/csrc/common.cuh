@@ -27,35 +27,20 @@ const unsigned long long* rng_offset_ptr();  // device counter added to every dr
 // Every kernel of this library starts with pdl_enter(): `launch_dependents` lets the NEXT kernel in the stream be
 // scheduled as soon as all CTAs of this one are resident (its CTAs fill SMs as ours retire, run their prologue and
 // park), `wait` then blocks until the PREVIOUS kernel has completed and flushed.  No global memory is touched before
-// the wait, so ordering is exactly that of a plain stream.  The launch attribute is only set with GB200_PDL=1:
-// inside the CUDA-graph replay of the C3 step, programmatic edges measured 4-8 % SLOWER than plain kernel edges
-// in every trigger placement tried (entry, after the MMAs, none), so the default is a plain launch.
-bool pdl_enabled();
-#ifndef GB200_PDL_MODE
-#define GB200_PDL_MODE 1     // 0: wait only; 1: trigger on kernel entry; 2: as 1, but the tcgen05 GEMM triggers when its MMAs are done
-#endif
-__device__ __forceinline__ void pdl_trigger_now() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void pdl_trigger() {
-    if (GB200_PDL_MODE != 0) pdl_trigger_now();
-}
+// the wait, so ordering is exactly that of a plain stream.  The library's own kernels are launched WITHOUT the
+// programmatic attribute: inside the CUDA-graph replay of the C3 step, programmatic edges measured 4-8 % SLOWER than
+// plain kernel edges in every trigger placement tried (entry, after the MMAs, none).  The entry trigger still matters:
+// the fused encoder chain (encoder_common.cuh) is launched with the attribute, and its first kernel starts early only
+// once the library kernel before it has triggered.
+__device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_enter() { pdl_trigger(); pdl_wait(); }
 
+// errors surface in check_launch()
 template <typename... KArgs, typename... Args>
-static inline void launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
-                              Args&&... args) {
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
-    cfg.gridDim = grid;
-    cfg.blockDim = block;
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = pdl_enabled() ? 1 : 0;
-    cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);   // errors surface in check_launch()
+static inline void launch_kernel(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
+                                 Args&&... args) {
+    kernel<<<grid, block, smem, st>>>(static_cast<KArgs>(args)...);
 }
 
 static inline int cdiv(long long a, long long b) { return (int)((a + b - 1) / b); }

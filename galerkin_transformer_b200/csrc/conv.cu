@@ -586,8 +586,7 @@ extern "C" int gb200_conv1_fwd(int device, const float* x, const float* w, float
     const long long total = (long long)B * H * W * (C / 4);
     int blocks = (int)((total + 255) / 256);
     if (blocks > 148 * 16) blocks = 148 * 16;
-    static const int rows_on = [] { const char* v = getenv("GB200_CONV1_ROWS"); return v ? atoi(v) : 1; }();
-    if (rows_on && C <= 128 && W <= 2048) {
+    if (C <= 128 && W <= 2048) {
         int rb = B * H;
         if (rb > 148 * 16) rb = 148 * 16;
         conv1_fwd_row_kernel<<<rb, 256, 3 * (W + 2) * sizeof(float), as_stream(stream)>>>(a);
@@ -615,8 +614,7 @@ extern "C" int gb200_conv1_bwd(int device, const float* dy, const float* y, cons
         ++launched;
     }
     int nparts = 148 * 4;
-    static const int rows_on = [] { const char* v = getenv("GB200_CONV1_ROWS"); return v ? atoi(v) : 1; }();
-    if (rows_on && W <= 512) {
+    if (W <= 512) {
         const int nrows = B * H;
         const int rpc = (nrows + nparts - 1) / nparts;          // the workspace holds 148 * 4 partials
         nparts = (nrows + rpc - 1) / rpc;

@@ -20,11 +20,6 @@ struct GemmEpilogue {
     const float* R; int ldr; float rscale;
     int accumulate;
     const float* G; int ldg; int gate;     // gate: ACT_RELU -> keep where G > 0; ACT_SILU -> times silu'(G); null = off
-    // fused per-head LayerNorm statistics (tcgen05 float4 epilogue only): columns [hn_lo, hn_hi) are split into
-    // groups of hn_dk; each group of a row is replaced by (v - mean) * rstd and rstd goes to hn_rstd[block][row, head]
-    int hn_dk, hn_lo, hn_hi, hn_heads;
-    float hn_eps;
-    float* hn_rstd[2];
 
     __device__ __forceinline__ void store(int batch, int m, int n, int M, int N, float acc) const {
         float v = alpha * acc;
@@ -80,9 +75,5 @@ struct GemmEpilogue {
         *c = v;
     }
 };
-
-// gate of the NEXT gb200_gemm / gb200_gemm_tc call on this thread (set by the *_gated entry points)
-struct GemmGate { const float* G; int ldg; int act; };
-GemmGate& next_gemm_gate();
 
 }  // namespace gb200

@@ -538,13 +538,12 @@ extern "C" int gb200_gemm_suggest_ksplit(int M, int N, int K, int nbatch) {
     return s < 1 ? 1 : (s > 128 ? 128 : s);
 }
 
-extern "C" int gb200_gemm(int device, const float* A, int lda, int transA, const float* B, int ldb,
-                          int transB, float* C, int ldc, int M, int N, int K, int nbatch,
-                          long long strideA, long long strideB, long long strideC, float alpha,
-                          const float* bias, int act, float* Zout, int ldz, float drop_p,
-                          unsigned long long seed, const float* R, int ldr, float rscale,
-                          int accumulate, int ksplit, float* workspace, size_t workspace_bytes,
-                          void* stream) {
+// gb200_gemm and gb200_gemm_gated: gate == nullptr is the plain GEMM
+static int gemm_simt(int device, const float* A, int lda, int transA, const float* B, int ldb, int transB, float* C,
+                     int ldc, int M, int N, int K, int nbatch, long long strideA, long long strideB, long long strideC,
+                     float alpha, const float* bias, int act, float* Zout, int ldz, float drop_p, unsigned long long seed,
+                     const float* R, int ldr, float rscale, int accumulate, const float* gate, int ldg, int gate_act,
+                     int ksplit, float* workspace, size_t workspace_bytes, void* stream) {
     use_device(device);
     GB_REQUIRE(M >= 0 && N >= 0 && K >= 0 && nbatch >= 1, "gb200_gemm: bad shape M=%d N=%d K=%d nb=%d", M, N, K, nbatch);
     if (M == 0 || N == 0) return GB200_OK;
@@ -561,10 +560,8 @@ extern "C" int gb200_gemm(int device, const float* A, int lda, int transA, const
     g.kchunk = cdiv(ktiles, ksplit) * BK;
     g.ep.alpha = alpha; g.ep.bias = bias; g.ep.act = act; g.ep.Z = Zout; g.ep.ldz = ldz; g.ep.drop_p = drop_p;
     g.ep.seed = seed; g.ep.seed_off = rng_offset_ptr(); g.ep.R = R; g.ep.ldr = ldr; g.ep.rscale = rscale; g.ep.accumulate = accumulate;
-    g.ep.hn_dk = 0; g.ep.hn_lo = g.ep.hn_hi = g.ep.hn_heads = 0; g.ep.hn_eps = 0.f; g.ep.hn_rstd[0] = g.ep.hn_rstd[1] = nullptr;
-    const GemmGate& gate = next_gemm_gate();
-    g.ep.G = gate.G; g.ep.ldg = gate.ldg; g.ep.gate = gate.act;
-    GB_REQUIRE(!gate.G || gate.act == ACT_RELU || gate.act == ACT_SILU, "gb200_gemm: unknown gate %d", gate.act);
+    g.ep.G = gate; g.ep.ldg = ldg; g.ep.gate = gate_act;
+    GB_REQUIRE(!gate || gate_act == ACT_RELU || gate_act == ACT_SILU, "gb200_gemm: unknown gate %d", gate_act);
     g.ws = workspace;
     g.vecA = ((uintptr_t)A % 16 == 0) && (lda % 4 == 0) && (strideA % 4 == 0);
     g.vecB = ((uintptr_t)B % 16 == 0) && (ldb % 4 == 0) && (strideB % 4 == 0);
@@ -588,61 +585,70 @@ extern "C" int gb200_gemm(int device, const float* A, int lda, int transA, const
         if (K <= 8 && total < (1ll << 31) && out4) {
             const long long quads = total / 4;
             const int blocks = (int)(quads / 256 + 1 < 148 * 16 ? quads / 256 + 1 : 148 * 16);
-            if (K <= 2) launch_pdl(gemm_thin_k_vec4_kernel<2>, blocks, 256, 0, st, s);
-            else launch_pdl(gemm_thin_k_vec4_kernel<8>, blocks, 256, 0, st, s);
+            if (K <= 2) launch_kernel(gemm_thin_k_vec4_kernel<2>, blocks, 256, 0, st, s);
+            else launch_kernel(gemm_thin_k_vec4_kernel<8>, blocks, 256, 0, st, s);
             return check_launch("gb200_gemm(thin K, float4)", 1);
         }
         if (K <= 8 && total < (1ll << 31)) {
-            launch_pdl(gemm_thin_k_kernel, (int)(total / 256 + 1 < 148 * 16 ? total / 256 + 1 : 148 * 16), 256, 0, st, s);
+            launch_kernel(gemm_thin_k_kernel, (int)(total / 256 + 1 < 148 * 16 ? total / 256 + 1 : 148 * 16), 256, 0, st, s);
             return check_launch("gb200_gemm(thin K)", 1);
         }
         if (N <= 2 && !transA && transB && M >= 1024 && K % 4 == 0 && al16(A) && al16(B) && lda % 4 == 0 && ldb % 4 == 0) {
             const int blocks = cdiv(M, 32) < 148 * 16 ? cdiv(M, 32) : 148 * 16;
-            if (N == 1) launch_pdl(gemm_thin_n_vec4_kernel<1>, blocks, 256, 0, st, s);
-            else launch_pdl(gemm_thin_n_vec4_kernel<2>, blocks, 256, 0, st, s);
+            if (N == 1) launch_kernel(gemm_thin_n_vec4_kernel<1>, blocks, 256, 0, st, s);
+            else launch_kernel(gemm_thin_n_vec4_kernel<2>, blocks, 256, 0, st, s);
             return check_launch("gb200_gemm(thin N, float4)", 1);
         }
         if (N <= 8 && !transA && M >= 1024) {
             const int blocks = cdiv(M, 8) < 148 * 16 ? cdiv(M, 8) : 148 * 16;
-            if (N <= 2) launch_pdl(gemm_thin_n_kernel<2>, blocks, 256, 0, st, s);
-            else launch_pdl(gemm_thin_n_kernel<8>, blocks, 256, 0, st, s);
+            if (N <= 2) launch_kernel(gemm_thin_n_kernel<2>, blocks, 256, 0, st, s);
+            else launch_kernel(gemm_thin_n_kernel<8>, blocks, 256, 0, st, s);
             return check_launch("gb200_gemm(thin N)", 1);
         }
         if (transA && !transB && total <= 1024 && ksplit > 1) {
             s.ksplit = cdiv(K, s.kchunk);
             if (N % 4 == 0 && total / 4 <= 256 && al16(B) && ldb % 4 == 0 && al16(workspace))
-                launch_pdl(gemm_tall_partial_vec4_kernel, s.ksplit, 256, 0, st, s);
+                launch_kernel(gemm_tall_partial_vec4_kernel, s.ksplit, 256, 0, st, s);
             else
-                launch_pdl(gemm_tall_partial_kernel, s.ksplit, 256, 0, st, s);
-            launch_pdl(gemm_tall_final_kernel, cdiv(total, 32), dim3(32, 32), 0, st, s);
+                launch_kernel(gemm_tall_partial_kernel, s.ksplit, 256, 0, st, s);
+            launch_kernel(gemm_tall_final_kernel, cdiv(total, 32), dim3(32, 32), 0, st, s);
             return check_launch("gb200_gemm(tall)", 2);
         }
     }
     dim3 grid(cdiv(N, BN), cdiv(M, BM), nbatch * ksplit);
     GB_REQUIRE(grid.y <= 65535 && grid.z <= 65535, "gb200_gemm: grid too large");
-    if (!transA && !transB) launch_pdl(gemm_simt_kernel<false, false>, grid, NT, 0, st, g);
-    else if (!transA && transB) launch_pdl(gemm_simt_kernel<false, true>, grid, NT, 0, st, g);
-    else if (transA && !transB) launch_pdl(gemm_simt_kernel<true, false>, grid, NT, 0, st, g);
-    else launch_pdl(gemm_simt_kernel<true, true>, grid, NT, 0, st, g);
+    if (!transA && !transB) launch_kernel(gemm_simt_kernel<false, false>, grid, NT, 0, st, g);
+    else if (!transA && transB) launch_kernel(gemm_simt_kernel<false, true>, grid, NT, 0, st, g);
+    else if (transA && !transB) launch_kernel(gemm_simt_kernel<true, false>, grid, NT, 0, st, g);
+    else launch_kernel(gemm_simt_kernel<true, true>, grid, NT, 0, st, g);
     if (ksplit > 1) {
         long long total = (long long)nbatch * M * N;
         int blocks = (int)((total + 255) / 256);
         if (blocks > 148 * 8) blocks = 148 * 8;
-        launch_pdl(splitk_reduce_kernel, blocks, 256, 0, st, g);
+        launch_kernel(splitk_reduce_kernel, blocks, 256, 0, st, g);
     }
     return check_launch("gb200_gemm", ksplit > 1 ? 2 : 1);
+}
+
+extern "C" int gb200_gemm(int device, const float* A, int lda, int transA, const float* B, int ldb,
+                          int transB, float* C, int ldc, int M, int N, int K, int nbatch,
+                          long long strideA, long long strideB, long long strideC, float alpha,
+                          const float* bias, int act, float* Zout, int ldz, float drop_p,
+                          unsigned long long seed, const float* R, int ldr, float rscale,
+                          int accumulate, int ksplit, float* workspace, size_t workspace_bytes,
+                          void* stream) {
+    return gemm_simt(device, A, lda, transA, B, ldb, transB, C, ldc, M, N, K, nbatch, strideA, strideB, strideC, alpha,
+                     bias, act, Zout, ldz, drop_p, seed, R, ldr, rscale, accumulate, nullptr, 0, ACT_NONE, ksplit,
+                     workspace, workspace_bytes, stream);
 }
 
 extern "C" int gb200_gemm_gated(int device, const float* A, int lda, int transA, const float* B, int ldb,
                                 int transB, float* C, int ldc, int M, int N, int K, float alpha, float drop_p,
                                 unsigned long long seed, float rscale, const float* gate, int ldg, int gate_act,
                                 int ksplit, float* workspace, size_t workspace_bytes, void* stream) {
-    GemmGate& gg = next_gemm_gate();
-    gg.G = gate; gg.ldg = ldg; gg.act = gate_act;
-    const int rc = gb200_gemm(device, A, lda, transA, B, ldb, transB, C, ldc, M, N, K, 1, 0, 0, 0, alpha, nullptr, ACT_NONE,
-                              nullptr, 0, drop_p, seed, nullptr, 0, rscale, 0, ksplit, workspace, workspace_bytes, stream);
-    gg.G = nullptr;
-    return rc;
+    return gemm_simt(device, A, lda, transA, B, ldb, transB, C, ldc, M, N, K, 1, 0, 0, 0, alpha, nullptr, ACT_NONE, nullptr,
+                     0, drop_p, seed, nullptr, 0, rscale, 0, gate, ldg, gate_act, ksplit, workspace, workspace_bytes,
+                     stream);
 }
 
 extern "C" size_t gb200_colsum_workspace_bytes(long long M, int N) {
@@ -661,9 +667,9 @@ extern "C" int gb200_colsum(int device, const float* X, int ld, long long M, int
                "gb200_colsum: workspace too small");
     GB_REQUIRE(nparts <= 65535, "gb200_colsum: too many rows");
     cudaStream_t st = as_stream(stream);
-    launch_pdl(colsum_partial_kernel, dim3(cdiv(N, 32), nparts), dim3(32, 32), 0, st, X, (int)M, N, ld, rows_per_block,
+    launch_kernel(colsum_partial_kernel, dim3(cdiv(N, 32), nparts), dim3(32, 32), 0, st, X, (int)M, N, ld, rows_per_block,
                                                                                workspace);
-    launch_pdl(colsum_final_kernel, cdiv(N, 32), dim3(32, 32), 0, st, workspace, nparts, N, scale, accumulate, out);
+    launch_kernel(colsum_final_kernel, cdiv(N, 32), dim3(32, 32), 0, st, workspace, nparts, N, scale, accumulate, out);
     return check_launch("gb200_colsum", 2);
 }
 
@@ -689,16 +695,16 @@ extern "C" int gb200_epilogue_bwd(int device, const float* dy, int lddy, const f
         float4* g4 = reinterpret_cast<float4*>(g);
         cudaStream_t st = as_stream(stream);
         if (act == ACT_RELU)
-            launch_pdl(epilogue_bwd_vec4_kernel<ACT_RELU>, blocks, 256, 0, st, d4, r4, g4, total4, rscale, drop_p, seed, rng_offset_ptr());
+            launch_kernel(epilogue_bwd_vec4_kernel<ACT_RELU>, blocks, 256, 0, st, d4, r4, g4, total4, rscale, drop_p, seed, rng_offset_ptr());
         else if (act == ACT_SILU)
-            launch_pdl(epilogue_bwd_vec4_kernel<ACT_SILU>, blocks, 256, 0, st, d4, r4, g4, total4, rscale, drop_p, seed, rng_offset_ptr());
+            launch_kernel(epilogue_bwd_vec4_kernel<ACT_SILU>, blocks, 256, 0, st, d4, r4, g4, total4, rscale, drop_p, seed, rng_offset_ptr());
         else
-            launch_pdl(epilogue_bwd_vec4_kernel<ACT_NONE>, blocks, 256, 0, st, d4, r4, g4, total4, rscale, drop_p, seed, rng_offset_ptr());
+            launch_kernel(epilogue_bwd_vec4_kernel<ACT_NONE>, blocks, 256, 0, st, d4, r4, g4, total4, rscale, drop_p, seed, rng_offset_ptr());
         return check_launch("gb200_epilogue_bwd");
     }
     int blocks = (int)((total + 255) / 256);
     if (blocks > 148 * 16) blocks = 148 * 16;
-    launch_pdl(epilogue_bwd_kernel, blocks, 256, 0, as_stream(stream), dy, lddy, z, ldz, y, ldy, g, ldg, M, N, act,
+    launch_kernel(epilogue_bwd_kernel, blocks, 256, 0, as_stream(stream), dy, lddy, z, ldz, y, ldy, g, ldg, M, N, act,
                                                                rscale, drop_p, seed, rng_offset_ptr());
     return check_launch("gb200_epilogue_bwd");
 }
@@ -739,14 +745,14 @@ extern "C" int gb200_epilogue_bwd_bias(int device, const float* dy, int lddy, co
     const float4* r4 = reinterpret_cast<const float4*>(ref);
     float4* g4 = reinterpret_cast<float4*>(g);
     if (act == ACT_RELU)
-        launch_pdl(epilogue_bwd_bias_kernel<ACT_RELU>, blocks, 256, 0, st, d4, r4, g4, (int)M, N, rscale, drop_p, seed,
+        launch_kernel(epilogue_bwd_bias_kernel<ACT_RELU>, blocks, 256, 0, st, d4, r4, g4, (int)M, N, rscale, drop_p, seed,
                                                                    rng_offset_ptr(), workspace);
     else if (act == ACT_SILU)
-        launch_pdl(epilogue_bwd_bias_kernel<ACT_SILU>, blocks, 256, 0, st, d4, r4, g4, (int)M, N, rscale, drop_p, seed,
+        launch_kernel(epilogue_bwd_bias_kernel<ACT_SILU>, blocks, 256, 0, st, d4, r4, g4, (int)M, N, rscale, drop_p, seed,
                                                                    rng_offset_ptr(), workspace);
     else
-        launch_pdl(epilogue_bwd_bias_kernel<ACT_NONE>, blocks, 256, 0, st, d4, r4, g4, (int)M, N, rscale, drop_p, seed,
+        launch_kernel(epilogue_bwd_bias_kernel<ACT_NONE>, blocks, 256, 0, st, d4, r4, g4, (int)M, N, rscale, drop_p, seed,
                                                                    rng_offset_ptr(), workspace);
-    launch_pdl(colsum_final_kernel, cdiv(N, 32), dim3(32, 32), 0, st, workspace, blocks, N, 1.f, 0, dbias);
+    launch_kernel(colsum_final_kernel, cdiv(N, 32), dim3(32, 32), 0, st, workspace, blocks, N, 1.f, 0, dbias);
     return check_launch("gb200_epilogue_bwd_bias", 2);
 }

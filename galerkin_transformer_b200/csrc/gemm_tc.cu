@@ -20,7 +20,6 @@
 //
 // All waits are bounded: a descriptor/protocol bug traps instead of hanging the device.
 #include <cuda.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 #include "gemm_epilogue.cuh"
@@ -36,17 +35,11 @@ constexpr int TC_BM = 128, TC_BK = 32, TC_THREADS = 192;
 // split (3xTF32) stages are twice as large: two of them keep the CTA under half an SM's shared memory for BN <= 64, so two
 // CTAs co-reside and one's prologue / epilogue overlaps the other's main loop (the tall-skinny decoder GEMMs are 8 waves of
 // single-tile CTAs: with one CTA per SM those phases were serialised, 62 us for a 16 us problem)
-#ifndef GB200_TC_STAGES_SPLIT
-#define GB200_TC_STAGES_SPLIT 2
-#endif
-#ifndef GB200_TC_STAGES_NARROW
-#define GB200_TC_STAGES_NARROW 4
-#endif
 // SPLIT ("3xTF32"): every operand tile also keeps its TF32 residual lo = rna(x - hi) in a second buffer and each k-step
 // issues hi.hi + hi.lo + lo.hi -- fp32-grade products (2^-22) for the forward / input-gradient GEMMs of 'x3' mode that no
 // fused kernel covers; stages are twice as large, so the ring is one stage shorter
 template <int BN, bool SPLIT = false> __host__ __device__ constexpr int tc_stages() {
-    return SPLIT ? GB200_TC_STAGES_SPLIT : (BN == 192 ? 2 : (BN <= 64 ? GB200_TC_STAGES_NARROW : 3));
+    return SPLIT ? 2 : (BN == 192 ? 2 : (BN <= 64 ? 4 : 3));
 }
 template <int BN> __host__ __device__ constexpr int tc_tmem_cols() { return BN == 192 ? 256 : BN; }     // power of two >= 32
 template <int BN, bool SPLIT = false> __host__ __device__ constexpr int tc_smem_bytes() {
@@ -60,7 +53,6 @@ struct TcArgs {
     int ksplit, kchunk;   // kchunk is a multiple of TC_BK
     float* ws;
     int vec4;             // C/R/Z/ws rows are 16-byte aligned and N % 4 == 0: float4 epilogue
-    int truncate;         // 1: skip the round-to-nearest pass (operands truncated to TF32 by the tensor core)
     unsigned long long* trace;   // diagnostics: 8 globaltimer stamps per CTA (gb200_gemm_tc_set_trace), else null
 };
 
@@ -85,7 +77,7 @@ __device__ __forceinline__ float act_fast(float v) {
 // Compile-time activation / dropout; residual, Z and accumulate are warp-uniform runtime switches.
 // GATE != 0 (host guarantees no residual / accumulate then): the rv registers carry the gate operand G instead and
 // v *= act'(G) before the dropout scale -- the elementwise backward between two Linear layers, fused.
-template <int ACT, bool DROP, bool HN = false, int GATE = 0>
+template <int ACT, bool DROP, int GATE = 0>
 __device__ __forceinline__ void tc_epilogue_vec4(const TcArgs& g, const float* __restrict__ stage, int DS, int lane,
                                                  int rbase, int n0, int ncols, unsigned long long seed) {
     const GemmEpilogue& ep = g.ep;
@@ -94,15 +86,10 @@ __device__ __forceinline__ void tc_epilogue_vec4(const TcArgs& g, const float* _
     const float alpha = ep.alpha, rscale = ep.rscale, p = ep.drop_p;
     const int nrows = min(32, g.M - rbase);
     const float4 zero4 = make_float4(0.f, 0.f, 0.f, 0.f);
-    // warp-uniform trip counts (the fused head-norm shuffles need every lane): columns past ncols are predicated
-    // (only the fused head-norm variant needs warp-uniform trip counts for its shuffles; the plain epilogue keeps the
-    // cheaper per-lane loop)
-    for (int cb = HN ? 0 : lane * 4; cb < ncols; cb += 128) {
-        const int c = HN ? cb + lane * 4 : cb;
-        const bool cv = HN ? (c < ncols) : true;
+    for (int c = lane * 4; c < ncols; c += 128) {
         const int n = n0 + c;
         float4 bv = zero4;
-        if (cv && ep.bias) bv = *reinterpret_cast<const float4*>(ep.bias + n);
+        if (ep.bias) bv = *reinterpret_cast<const float4*>(ep.bias + n);
         const float* rp = GATE ? ep.G + (long long)rbase * ep.ldg + n : (hasR ? ep.R + (long long)rbase * ep.ldr + n : nullptr);
         const int ldr = GATE ? ep.ldg : ep.ldr;
         float* cp = ep.C + (long long)rbase * ep.ldc + n;
@@ -112,9 +99,9 @@ __device__ __forceinline__ void tc_epilogue_vec4(const TcArgs& g, const float* _
             float4 acc[RB], rv[RB];
 #pragma unroll
             for (int i = 0; i < RB; ++i) {
-                acc[i] = cv ? *reinterpret_cast<const float4*>(&stage[(r0 + i) * DS + c]) : zero4;
+                acc[i] = *reinterpret_cast<const float4*>(&stage[(r0 + i) * DS + c]);
                 rv[i] = zero4;
-                if (cv && r0 + i < nrows) {
+                if (r0 + i < nrows) {
                     if (GATE || hasR) rv[i] = *reinterpret_cast<const float4*>(rp + (long long)(r0 + i) * ldr);
                     if (!GATE && accum) {
                         const float4 cvv = *reinterpret_cast<const float4*>(cp + (long long)(r0 + i) * ep.ldc);
@@ -127,29 +114,6 @@ __device__ __forceinline__ void tc_epilogue_vec4(const TcArgs& g, const float* _
                 if (r0 + i >= nrows) break;                                  // uniform across the warp
                 float4 z = make_float4(fmaf(alpha, acc[i].x, bv.x), fmaf(alpha, acc[i].y, bv.y),
                                        fmaf(alpha, acc[i].z, bv.z), fmaf(alpha, acc[i].w, bv.w));
-                if (HN) {
-                    // per-head LayerNorm statistics over the hn_dk columns of this row's head group (hn_dk / 4 lanes)
-                    const int lg = ep.hn_dk >> 2;
-                    float sm = z.x + z.y + z.z + z.w;
-#pragma unroll
-                    for (int o = 16; o > 0; o >>= 1)
-                        if (o < lg) sm += __shfl_xor_sync(0xffffffffu, sm, o);      // lg is warp-uniform
-                    const float mean = sm / ep.hn_dk;
-                    const float dx = z.x - mean, dy = z.y - mean, dz = z.z - mean, dw = z.w - mean;
-                    float sq = dx * dx + dy * dy + dz * dz + dw * dw;
-#pragma unroll
-                    for (int o = 16; o > 0; o >>= 1)
-                        if (o < lg) sq += __shfl_xor_sync(0xffffffffu, sq, o);
-                    const float rs = rsqrtf(sq / ep.hn_dk + ep.hn_eps);
-                    if (cv && n >= ep.hn_lo && n < ep.hn_hi) {
-                        z = make_float4(dx * rs, dy * rs, dz * rs, dw * rs);
-                        if ((lane & (lg - 1)) == 0) {
-                            const int rel = n - ep.hn_lo, blkw = ep.hn_heads * ep.hn_dk;
-                            ep.hn_rstd[rel / blkw][(long long)(rbase + r0 + i) * ep.hn_heads + (rel % blkw) / ep.hn_dk] = rs;
-                        }
-                    }
-                }
-                if (!cv) continue;
                 if (hasZ) *reinterpret_cast<float4*>(zp + (long long)(r0 + i) * ep.ldz) = z;
                 float4 v = make_float4(act_fast<ACT>(z.x), act_fast<ACT>(z.y), act_fast<ACT>(z.z), act_fast<ACT>(z.w));
                 if (GATE == ACT_RELU) {
@@ -195,7 +159,7 @@ __device__ __forceinline__ void gemm_tc_body(const CUtensorMap& mapA, const CUte
     const int kbeg = split * g.kchunk;
     const int kend = min(g.K, kbeg + g.kchunk);
     const int nkb = (kend - kbeg + TC_BK - 1) / TC_BK;
-    if (GB200_PDL_MODE == 1) pdl_trigger_now();
+    pdl_trigger();
     if (threadIdx.x == 64) tc_stamp(g, 0);                                   // CTA entry
 
     if (threadIdx.x == 0) {
@@ -259,7 +223,7 @@ __device__ __forceinline__ void gemm_tc_body(const CUtensorMap& mapA, const CUte
             for (int kb = 0; kb < nkb; ++kb) {
                 const int s = kb % TC_STAGES;
                 const uint32_t ph = (kb / TC_STAGES) & 1;
-                mbar_wait((g.truncate && !SPLIT) ? &full_bar[s] : &conv_bar[s], ph);   // tile landed (TMA) [and rounded to TF32]
+                mbar_wait(&conv_bar[s], ph);     // tile landed (TMA) and rounded to TF32
                 tc_fence_after();
                 const uint32_t sa = smem_u32(smem + s * STAGE_BYTES);
                 const uint32_t sb = sa + A_BYTES;
@@ -293,7 +257,7 @@ __device__ __forceinline__ void gemm_tc_body(const CUtensorMap& mapA, const CUte
         // systematic -1e-3 relative bias per product); rounding makes the error zero-mean like cuBLAS TF32.
         {
             const int ct = threadIdx.x - 64;     // 0..127
-            for (int kb = 0; kb < ((g.truncate && !SPLIT) ? 0 : nkb); ++kb) {
+            for (int kb = 0; kb < nkb; ++kb) {
                 const int s = kb % TC_STAGES;
                 const uint32_t ph = (kb / TC_STAGES) & 1;
                 mbar_wait(&full_bar[s], ph);
@@ -337,7 +301,6 @@ __device__ __forceinline__ void gemm_tc_body(const CUtensorMap& mapA, const CUte
             tc_fence_after();
         }
         if (threadIdx.x == 64) tc_stamp(g, 5);                               // accumulator complete
-        if (GB200_PDL_MODE == 2 && threadIdx.x == 64) pdl_trigger_now();
 #pragma unroll 1
         for (int c0 = 0; c0 < BN; c0 += 32) {
             uint32_t v[32];
@@ -382,15 +345,13 @@ __device__ __forceinline__ void gemm_tc_body(const CUtensorMap& mapA, const CUte
                         *reinterpret_cast<const float4*>(&stage[r * DS + c]);
         } else if (g.vec4) {
             const bool drop = ep.drop_p > 0.f;
-            if (ep.hn_dk) {        // QKV projection with fused per-head LayerNorm (host guarantees act none, no dropout)
-                tc_epilogue_vec4<ACT_NONE, false, true>(g, stage, DS, lane, rbase, n0, ncols, seed);
-            } else if (ep.G) {     // gated backward GEMM (host guarantees act none, no residual / accumulate)
+            if (ep.G) {     // gated backward GEMM (host guarantees act none, no residual / accumulate)
                 if (ep.gate == ACT_RELU) {
-                    if (drop) tc_epilogue_vec4<ACT_NONE, true, false, ACT_RELU>(g, stage, DS, lane, rbase, n0, ncols, seed);
-                    else tc_epilogue_vec4<ACT_NONE, false, false, ACT_RELU>(g, stage, DS, lane, rbase, n0, ncols, seed);
+                    if (drop) tc_epilogue_vec4<ACT_NONE, true, ACT_RELU>(g, stage, DS, lane, rbase, n0, ncols, seed);
+                    else tc_epilogue_vec4<ACT_NONE, false, ACT_RELU>(g, stage, DS, lane, rbase, n0, ncols, seed);
                 } else {
-                    if (drop) tc_epilogue_vec4<ACT_NONE, true, false, ACT_SILU>(g, stage, DS, lane, rbase, n0, ncols, seed);
-                    else tc_epilogue_vec4<ACT_NONE, false, false, ACT_SILU>(g, stage, DS, lane, rbase, n0, ncols, seed);
+                    if (drop) tc_epilogue_vec4<ACT_NONE, true, ACT_SILU>(g, stage, DS, lane, rbase, n0, ncols, seed);
+                    else tc_epilogue_vec4<ACT_NONE, false, ACT_SILU>(g, stage, DS, lane, rbase, n0, ncols, seed);
                 }
             } else if (ep.act == ACT_NONE) {
                 if (drop) tc_epilogue_vec4<ACT_NONE, true>(g, stage, DS, lane, rbase, n0, ncols, seed);
@@ -507,31 +468,29 @@ __global__ void tc_splitk_reduce_group_kernel(const __grid_constant__ TcGroup G)
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// Persistent variant (ksplit == 1): one CTA per SM walks a static list of output tiles.  The shared-memory ring
-// (4 stages) runs continuously across tile boundaries and the accumulator is double-buffered in TMEM, so the
-// epilogue of tile i (TMEM -> smem -> global) overlaps the TMA / convert / MMA work of tile i+1, and the fixed
-// per-CTA costs (barrier init, TMEM allocation, tensor-map fetch) are paid once per SM instead of once per tile.
+// Persistent variant for split (3xTF32) GEMMs with a K-major A and ksplit == 1: one CTA per SM walks a static list of
+// output tiles.  The shared-memory ring runs continuously across tile boundaries and the accumulator is double-buffered
+// in TMEM, so the epilogue of tile i (TMEM -> smem -> global) overlaps the TMA / convert / MMA work of tile i+1, and the
+// fixed per-CTA costs (barrier init, TMEM allocation, tensor-map fetch) are paid once per SM instead of once per tile.
 //   warp 0: TMA producer | warp 1: MMA issuer | warps 2-5: TF32 round-to-nearest converters |
 //   warps 6-13: epilogue (two warps per 32-lane TMEM quarter, each taking half of the tile's columns)
 // ---------------------------------------------------------------------------------------------------------
 constexpr int TCP_EPI_WARPS = 8, TCP_THREADS = (6 + TCP_EPI_WARPS) * 32;
-// ring depth: as many stages as fit beside the epilogue staging tile; split (3xTF32) stages carry a hi and a lo copy
-template <int BN, bool SPLIT> __host__ __device__ constexpr int tcp_stages() {
-    return !SPLIT ? 4 : (BN <= 32 ? 4 : (BN <= 64 ? 3 : 2));
-}
-template <int BN, bool SPLIT> __host__ __device__ constexpr int tcp_smem_bytes() {
-    return tcp_stages<BN, SPLIT>() * (SPLIT ? 2 : 1) * (TC_BM * TC_BK * 4 + BN * TC_BK * 4) + TC_BM * (BN + 4) * 4 + 1024 + 256;
+// ring depth: as many stages as fit beside the epilogue staging tile; every stage carries a hi and a lo copy
+template <int BN> __host__ __device__ constexpr int tcp_stages() { return BN <= 32 ? 4 : (BN <= 64 ? 3 : 2); }
+template <int BN> __host__ __device__ constexpr int tcp_smem_bytes() {
+    return tcp_stages<BN>() * 2 * (TC_BM * TC_BK * 4 + BN * TC_BK * 4) + TC_BM * (BN + 4) * 4 + 1024 + 256;
 }
 
-template <int BN, bool A_MN, bool B_MN, bool SPLIT = false>
+template <int BN, bool B_MN>
 __global__ void __launch_bounds__(TCP_THREADS, 1) gemm_tc_persistent_kernel(const __grid_constant__ CUtensorMap mapA,
                                                                             const __grid_constant__ CUtensorMap mapB,
                                                                             TcArgs g) {
     constexpr int A_BYTES = TC_BM * TC_BK * 4;
     constexpr int B_BYTES = BN * TC_BK * 4;
     constexpr int TILE_PAIR = A_BYTES + B_BYTES;               // what TMA lands per k-block
-    constexpr int STAGE_BYTES = (SPLIT ? 2 : 1) * TILE_PAIR;   // SPLIT: [A hi | B hi | A lo | B lo]
-    constexpr int TCP_STAGES = tcp_stages<BN, SPLIT>();
+    constexpr int STAGE_BYTES = 2 * TILE_PAIR;                 // [A hi | B hi | A lo | B lo]
+    constexpr int TCP_STAGES = tcp_stages<BN>();
     constexpr int DS = BN + 4;
     constexpr int TMEM_COLS = 2 * BN < 32 ? 32 : 2 * BN;      // two accumulator buffers (power of two >= 32)
     extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -589,12 +548,7 @@ __global__ void __launch_bounds__(TCP_THREADS, 1) gemm_tc_persistent_kernel(cons
                     uint8_t* sb = sa + A_BYTES;
                     mbar_expect_tx(&full_bar[s], TILE_PAIR);
                     const int k0 = kb * TC_BK;
-                    if (!A_MN) {
-                        tma_load_2d(sa, &mapA, &full_bar[s], k0, m0);
-                    } else {
-#pragma unroll
-                        for (int j = 0; j < TC_BM / 32; ++j) tma_load_2d(sa + j * 4096, &mapA, &full_bar[s], m0 + 32 * j, k0);
-                    }
+                    tma_load_2d(sa, &mapA, &full_bar[s], k0, m0);
                     if (!B_MN) {
                         tma_load_2d(sb, &mapB, &full_bar[s], k0, n0);
                     } else {
@@ -606,9 +560,8 @@ __global__ void __launch_bounds__(TCP_THREADS, 1) gemm_tc_persistent_kernel(cons
         }
     } else if (warp == 1) {
         if (lane == 0) {   // ---------------- MMA issuer ----------------
-            const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((A_MN ? 1u : 0u) << 15) |
-                                   ((B_MN ? 1u : 0u) << 16) | ((uint32_t)(BN >> 3) << 17) |
-                                   ((uint32_t)(TC_BM >> 4) << 24);
+            const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((B_MN ? 1u : 0u) << 16) |
+                                   ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(TC_BM >> 4) << 24);
             uint32_t it = 0, j = 0;
             for (int t = blockIdx.x; t < ntiles; t += gridDim.x, ++j) {
                 const uint32_t buf = j & 1;
@@ -624,16 +577,14 @@ __global__ void __launch_bounds__(TCP_THREADS, 1) gemm_tc_persistent_kernel(cons
                     const uint32_t sb = sa + A_BYTES;
 #pragma unroll
                     for (int k = 0; k < TC_BK / 8; ++k) {
-                        const uint64_t ad = A_MN ? umma_desc<1>(sa + k * 1024, 4096, 512) : umma_desc<2>(sa + k * 32, 16, 1024);
+                        const uint64_t ad = umma_desc<2>(sa + k * 32, 16, 1024);
                         const uint64_t bd = B_MN ? umma_desc<1>(sb + k * 1024, 4096, 512) : umma_desc<2>(sb + k * 32, 16, 1024);
                         tc_mma_tf32(tacc, ad, bd, idesc, (kb | k) != 0);
-                        if (SPLIT) {
-                            const uint32_t la = sa + TILE_PAIR, lb = sb + TILE_PAIR;
-                            const uint64_t adl = A_MN ? umma_desc<1>(la + k * 1024, 4096, 512) : umma_desc<2>(la + k * 32, 16, 1024);
-                            const uint64_t bdl = B_MN ? umma_desc<1>(lb + k * 1024, 4096, 512) : umma_desc<2>(lb + k * 32, 16, 1024);
-                            tc_mma_tf32(tacc, ad, bdl, idesc, 1u);
-                            tc_mma_tf32(tacc, adl, bd, idesc, 1u);
-                        }
+                        const uint32_t la = sa + TILE_PAIR, lb = sb + TILE_PAIR;       // residual (lo) copies
+                        const uint64_t adl = umma_desc<2>(la + k * 32, 16, 1024);
+                        const uint64_t bdl = B_MN ? umma_desc<1>(lb + k * 1024, 4096, 512) : umma_desc<2>(lb + k * 32, 16, 1024);
+                        tc_mma_tf32(tacc, ad, bdl, idesc, 1u);
+                        tc_mma_tf32(tacc, adl, bd, idesc, 1u);
                     }
                     tc_commit(&empty_bar[s]);
                 }
@@ -659,15 +610,14 @@ __global__ void __launch_bounds__(TCP_THREADS, 1) gemm_tc_persistent_kernel(cons
                     asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(w) : "f"(v.w));
                     tile[i] = make_float4(__uint_as_float(x), __uint_as_float(y), __uint_as_float(z),
                                           __uint_as_float(w));
-                    if (SPLIT) {       // residual, itself rounded to TF32 (same swizzled position in the lo copy)
-                        uint32_t a, b, c, d;
-                        asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(a) : "f"(v.x - __uint_as_float(x)));
-                        asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(b) : "f"(v.y - __uint_as_float(y)));
-                        asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(c) : "f"(v.z - __uint_as_float(z)));
-                        asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(d) : "f"(v.w - __uint_as_float(w)));
-                        tile[i + TILE_PAIR / 16] = make_float4(__uint_as_float(a), __uint_as_float(b), __uint_as_float(c),
-                                                               __uint_as_float(d));
-                    }
+                    // residual, itself rounded to TF32 (same swizzled position in the lo copy)
+                    uint32_t a, b, c, d;
+                    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(a) : "f"(v.x - __uint_as_float(x)));
+                    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(b) : "f"(v.y - __uint_as_float(y)));
+                    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(c) : "f"(v.z - __uint_as_float(z)));
+                    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(d) : "f"(v.w - __uint_as_float(w)));
+                    tile[i + TILE_PAIR / 16] = make_float4(__uint_as_float(a), __uint_as_float(b), __uint_as_float(c),
+                                                           __uint_as_float(d));
                 }
                 asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
                 __syncwarp();
@@ -724,11 +674,11 @@ __global__ void __launch_bounds__(TCP_THREADS, 1) gemm_tc_persistent_kernel(cons
                     const bool drop = ep.drop_p > 0.f;
                     if (ep.G) {            // gated backward GEMM (host guarantees act none, no residual / accumulate)
                         if (ep.gate == ACT_RELU) {
-                            if (drop) tc_epilogue_vec4<ACT_NONE, true, false, ACT_RELU>(g, stage, DS, lane, rbase, nc0, ncols, seed);
-                            else tc_epilogue_vec4<ACT_NONE, false, false, ACT_RELU>(g, stage, DS, lane, rbase, nc0, ncols, seed);
+                            if (drop) tc_epilogue_vec4<ACT_NONE, true, ACT_RELU>(g, stage, DS, lane, rbase, nc0, ncols, seed);
+                            else tc_epilogue_vec4<ACT_NONE, false, ACT_RELU>(g, stage, DS, lane, rbase, nc0, ncols, seed);
                         } else {
-                            if (drop) tc_epilogue_vec4<ACT_NONE, true, false, ACT_SILU>(g, stage, DS, lane, rbase, nc0, ncols, seed);
-                            else tc_epilogue_vec4<ACT_NONE, false, false, ACT_SILU>(g, stage, DS, lane, rbase, nc0, ncols, seed);
+                            if (drop) tc_epilogue_vec4<ACT_NONE, true, ACT_SILU>(g, stage, DS, lane, rbase, nc0, ncols, seed);
+                            else tc_epilogue_vec4<ACT_NONE, false, ACT_SILU>(g, stage, DS, lane, rbase, nc0, ncols, seed);
                         }
                     } else if (ep.act == ACT_NONE) {
                         if (drop) tc_epilogue_vec4<ACT_NONE, true>(g, stage, DS, lane, rbase, nc0, ncols, seed);
@@ -795,17 +745,17 @@ static int launch_tc(const CUtensorMap& ma, const CUtensorMap& mb, const TcArgs&
         configured = true;
     }
     dim3 grid(cdiv(g.N, BN), cdiv(g.M, TC_BM), g.ksplit);
-    launch_pdl(gemm_tc_kernel<BN, A_MN, B_MN, SPLIT>, grid, TC_THREADS, smem, st, ma, mb, g);
+    launch_kernel(gemm_tc_kernel<BN, A_MN, B_MN, SPLIT>, grid, TC_THREADS, smem, st, ma, mb, g);
     return 0;
 }
 
-template <int BN, bool A_MN, bool B_MN, bool SPLIT = false>
+template <int BN, bool B_MN>
 static int launch_tc_persistent(const CUtensorMap& ma, const CUtensorMap& mb, const TcArgs& g, cudaStream_t st) {
-    constexpr int smem = tcp_smem_bytes<BN, SPLIT>();
+    constexpr int smem = tcp_smem_bytes<BN>();
     static_assert(smem <= 232448, "persistent GEMM: shared memory");
     static bool configured = false;
     if (!configured) {
-        cudaFuncSetAttribute(gemm_tc_persistent_kernel<BN, A_MN, B_MN, SPLIT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+        cudaFuncSetAttribute(gemm_tc_persistent_kernel<BN, B_MN>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
         configured = true;
     }
     static int num_sms = 0;
@@ -817,7 +767,7 @@ static int launch_tc_persistent(const CUtensorMap& ma, const CUtensorMap& mb, co
     }
     const int tiles = cdiv(g.N, BN) * cdiv(g.M, TC_BM);
     const int grid = tiles < num_sms ? tiles : num_sms;
-    launch_pdl(gemm_tc_persistent_kernel<BN, A_MN, B_MN, SPLIT>, grid, TCP_THREADS, smem, st, ma, mb, g);
+    launch_kernel(gemm_tc_persistent_kernel<BN, B_MN>, grid, TCP_THREADS, smem, st, ma, mb, g);
     return 0;
 }
 
@@ -832,17 +782,9 @@ extern "C" int gb200_gemm_tc_supported(const float* A, int lda, const float* B, 
 }
 
 // widest N tile that still gives every SM a CTA (two co-reside per SM); narrow outputs get narrow tiles
-static int env_int(const char* name, int dflt) {
-    const char* v = getenv(name);
-    return v ? atoi(v) : dflt;
-}
-
 static int pick_bn(int M, int N) {
-    static const int forced = env_int("GB200_TC_BN", 0);        // tuning override (tools/bench_gemm.py)
-    if (forced && N >= forced) return forced;
     const long long mt = cdiv(M, TC_BM);
-    static const int wide = env_int("GB200_TC_BN192", 1);
-    if (wide && N >= 192 && N % 192 == 0 && mt * cdiv(N, 128) > 2 * 148 && mt * (N / 192) <= 2 * 148)
+    if (N >= 192 && N % 192 == 0 && mt * cdiv(N, 128) > 2 * 148 && mt * (N / 192) <= 2 * 148)
         return 192;      // one resident wave instead of two (the Q|K|V projection at C3: 232 CTAs, not 348)
     if (N >= 128 && mt * cdiv(N, 128) >= 148) return 128;
     if (N >= 64 && mt * cdiv(N, 64) >= 148) return 64;
@@ -855,39 +797,24 @@ extern "C" int gb200_gemm_tc_suggest_ksplit(int M, int N, int K) {
     long long tiles = (long long)cdiv(M, TC_BM) * cdiv(N, bn);
     if (tiles >= 120 || K < 1024) return 1;
     int want = (int)((2 * 148 + tiles - 1) / tiles);
-    static const int kdiv = env_int("GB200_TC_KSPLIT_DIV", 256);   // min K per split (tuning override)
-    int maxs = K / kdiv;
+    int maxs = K / 256;                  // at least 256 of K per split
     int s = want < maxs ? want : maxs;
     return s < 1 ? 1 : (s > 64 ? 64 : s);
 }
 
 namespace gb200 {
-struct HeadNormFusion { int dk, lo, hi, heads; float eps; float* rstd[2]; };
 static unsigned long long* g_tc_trace = nullptr;
 extern "C" int gb200_gemm_tc_set_trace(unsigned long long* device_buffer) {
     g_tc_trace = device_buffer;
     return 0;
 }
 
-static thread_local HeadNormFusion g_hn = {0, 0, 0, 0, 0.f, {nullptr, nullptr}};
-static thread_local int g_split_next = 0;
-}
-
-/* The NEXT gb200_gemm_tc / gb200_gemm_tc_gated call on this thread runs in split ("3xTF32") arithmetic: each product is
- * hi.hi + hi.lo + lo.hi of the TF32 two-term split of its fp32 operands (~2^-22 relative).  One-shot. */
-extern "C" int gb200_gemm_tc_split_next(int on) {
-    g_split_next = on;
-    return 0;
-}
-
-extern "C" int gb200_gemm_tc(int device, const float* A, int lda, int transA, const float* B, int ldb, int transB,
-                             float* C, int ldc, int M, int N, int K, float alpha, const float* bias, int act,
-                             float* Zout, int ldz, float drop_p, unsigned long long seed, const float* R, int ldr,
-                             float rscale, int accumulate, int ksplit, float* workspace, size_t workspace_bytes,
-                             void* stream) {
+// gb200_gemm_tc and gb200_gemm_tc_gated: gate == nullptr is the plain GEMM
+static int gemm_tc(int device, const float* A, int lda, int transA, const float* B, int ldb, int transB, float* C, int ldc,
+                   int M, int N, int K, float alpha, const float* bias, int act, float* Zout, int ldz, float drop_p,
+                   unsigned long long seed, const float* R, int ldr, float rscale, int accumulate, const float* gate, int ldg,
+                   int gate_act, int ksplit, float* workspace, size_t workspace_bytes, int split, void* stream) {
     use_device(device);
-    const bool split = g_split_next != 0;      // one-shot, consumed even if this call fails validation
-    g_split_next = 0;
     GB_REQUIRE(A && B && C, "gb200_gemm_tc: null operand");
     GB_REQUIRE(gb200_gemm_tc_supported(A, lda, B, ldb, M, N, K),
                "gb200_gemm_tc: unsupported shape/alignment (M=%d N=%d K=%d lda=%d ldb=%d); use gb200_gemm", M, N, K,
@@ -902,12 +829,9 @@ extern "C" int gb200_gemm_tc(int device, const float* A, int lda, int transA, co
     g.ep.C = C; g.ep.ldc = ldc; g.ep.sC = 0; g.ep.alpha = alpha; g.ep.bias = bias; g.ep.act = act; g.ep.Z = Zout;
     g.ep.ldz = ldz; g.ep.drop_p = drop_p; g.ep.seed = seed; g.ep.seed_off = rng_offset_ptr(); g.trace = g_tc_trace; g.ep.R = R; g.ep.ldr = ldr; g.ep.rscale = rscale;
     g.ep.accumulate = accumulate;
-    const GemmGate& gate = next_gemm_gate();
-    g.ep.G = gate.G; g.ep.ldg = gate.ldg; g.ep.gate = gate.act;
-    GB_REQUIRE(!gate.G || ((gate.act == ACT_RELU || gate.act == ACT_SILU) && act == ACT_NONE && !g_hn.dk),
-               "gb200_gemm_tc: bad gate (act %d)", gate.act);
-    g.ep.hn_dk = g_hn.dk; g.ep.hn_lo = g_hn.lo; g.ep.hn_hi = g_hn.hi; g.ep.hn_heads = g_hn.heads; g.ep.hn_eps = g_hn.eps;
-    g.ep.hn_rstd[0] = g_hn.rstd[0]; g.ep.hn_rstd[1] = g_hn.rstd[1];
+    g.ep.G = gate; g.ep.ldg = ldg; g.ep.gate = gate_act;
+    GB_REQUIRE(!gate || ((gate_act == ACT_RELU || gate_act == ACT_SILU) && act == ACT_NONE),
+               "gb200_gemm_tc: bad gate (act %d)", gate_act);
     g.M = M; g.N = N; g.K = K; g.ksplit = ksplit;
     g.kchunk = cdiv(cdiv(K, TC_BK), ksplit) * TC_BK;
     g.ksplit = cdiv(K, g.kchunk);
@@ -915,95 +839,75 @@ extern "C" int gb200_gemm_tc(int device, const float* A, int lda, int transA, co
     auto al16 = [](const void* p) { return ((uintptr_t)p % 16) == 0; };
     g.vec4 = (N % 4 == 0) && al16(C) && (ldc % 4 == 0) && (!R || (al16(R) && ldr % 4 == 0)) &&
              (!Zout || (al16(Zout) && ldz % 4 == 0)) && (!bias || al16(bias)) && (!workspace || al16(workspace)) &&
-             (!gate.G || (al16(gate.G) && gate.ldg % 4 == 0 && !R && !accumulate));
+             (!gate || (al16(gate) && ldg % 4 == 0 && !R && !accumulate));
     if (g.ksplit > 1)
         GB_REQUIRE(workspace && workspace_bytes >= (size_t)g.ksplit * M * N * sizeof(float),
                    "gb200_gemm_tc: split-K workspace too small");
-    GB_REQUIRE(!g.ep.hn_dk || (g.vec4 && g.ksplit == 1), "gb200_gemm_tc: fused head-norm needs the float4 epilogue");
-    static const int use_persistent = env_int("GB200_TC_PERSISTENT", 0);   // measured equal/slower in the full step
     // split (3xTF32) tall-skinny problems -- the decoder's per-pixel linears, 1243 row tiles of a K <= 130 GEMM -- are bound by
     // per-tile latency (prologue, first TMA, epilogue) in the one-tile-per-CTA kernel: the persistent kernel keeps the ring
-    // streaming across tiles and drains tile i while tile i+1 is loading
-    static const int split_persistent = env_int("GB200_TC_SPLIT_PERSISTENT", 1);
-    const bool sp = split && split_persistent && !a_mn && g.ksplit == 1 && !g.ep.hn_dk && g.vec4 &&
-                    (long long)cdiv(M, TC_BM) * cdiv(N, 128) >= 2 * 148;
-    const bool persistent = sp || (use_persistent && !split && g.ksplit == 1 && !g.ep.hn_dk && !g.ep.G);
-    if (bn == 192 && (persistent || g.ep.hn_dk || split)) bn = 128;
-    static const int split_bn_cap = env_int("GB200_TC_SPLIT_BN", 64);
-    if (split && !persistent && bn > split_bn_cap && (long long)cdiv(M, TC_BM) * cdiv(N, split_bn_cap) >= 2 * 148) bn = split_bn_cap;
-    if (sp) bn = N >= 128 ? 128 : (N >= 64 ? 64 : 32);
+    // streaming across tiles and drains tile i while tile i+1 is loading.  For single-pass TF32 it measured equal or slower
+    // in the full step, so only split problems take it.
+    const bool persistent = split && !a_mn && g.ksplit == 1 && g.vec4 && (long long)cdiv(M, TC_BM) * cdiv(N, 128) >= 2 * 148;
+    if (bn == 192 && split) bn = 128;
+    if (split && !persistent && bn > 64 && (long long)cdiv(M, TC_BM) * cdiv(N, 64) >= 2 * 148) bn = 64;
+    if (persistent) bn = N >= 128 ? 128 : (N >= 64 ? 64 : 32);
     CUtensorMap ma, mb;
     const CUtensorMapSwizzle SWK = CU_TENSOR_MAP_SWIZZLE_128B, SWMN = CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B;
     bool ok = a_mn ? make_map(&ma, A, M, K, lda, 32, 32, SWMN) : make_map(&ma, A, K, M, lda, 32, TC_BM, SWK);
     ok = ok && (b_mn ? make_map(&mb, B, N, K, ldb, 32, 32, SWMN) : make_map(&mb, B, K, N, ldb, 32, bn, SWK));
     GB_REQUIRE(ok, "gb200_gemm_tc: cuTensorMapEncodeTiled failed (M=%d N=%d K=%d lda=%d ldb=%d)", M, N, K, lda, ldb);
     cudaStream_t st = as_stream(stream);
-    static const int truncate = env_int("GB200_TC_TRUNCATE", 0);
-    g.truncate = truncate;
-#define TC_DISPATCH(BNV)                                                                          \
-    do {                                                                                          \
-        if (persistent) {                                                                         \
-            if (!a_mn && !b_mn) launch_tc_persistent<BNV, false, false>(ma, mb, g, st);           \
-            else if (!a_mn && b_mn) launch_tc_persistent<BNV, false, true>(ma, mb, g, st);        \
-            else if (a_mn && !b_mn) launch_tc_persistent<BNV, true, false>(ma, mb, g, st);        \
-            else launch_tc_persistent<BNV, true, true>(ma, mb, g, st);                            \
-        } else {                                                                                  \
-            if (!a_mn && !b_mn) launch_tc<BNV, false, false>(ma, mb, g, st);                      \
-            else if (!a_mn && b_mn) launch_tc<BNV, false, true>(ma, mb, g, st);                   \
-            else if (a_mn && !b_mn) launch_tc<BNV, true, false>(ma, mb, g, st);                   \
-            else launch_tc<BNV, true, true>(ma, mb, g, st);                                       \
-        }                                                                                         \
+#define TC_LAYOUT(BNV, SPLITV)                                                             \
+    do {                                                                                   \
+        if (!a_mn && !b_mn) launch_tc<BNV, false, false, SPLITV>(ma, mb, g, st);          \
+        else if (!a_mn && b_mn) launch_tc<BNV, false, true, SPLITV>(ma, mb, g, st);       \
+        else if (a_mn && !b_mn) launch_tc<BNV, true, false, SPLITV>(ma, mb, g, st);       \
+        else launch_tc<BNV, true, true, SPLITV>(ma, mb, g, st);                           \
     } while (0)
-    if (sp) {
-#define TC_SPLIT_P(BNV)                                                                         \
-    do {                                                                                        \
-        if (!b_mn) launch_tc_persistent<BNV, false, false, true>(ma, mb, g, st);                \
-        else launch_tc_persistent<BNV, false, true, true>(ma, mb, g, st);                       \
+#define TC_PERSISTENT(BNV)                                                                 \
+    do {                                                                                   \
+        if (!b_mn) launch_tc_persistent<BNV, false>(ma, mb, g, st);                        \
+        else launch_tc_persistent<BNV, true>(ma, mb, g, st);                               \
     } while (0)
-        if (bn == 128) TC_SPLIT_P(128);
-        else if (bn == 64) TC_SPLIT_P(64);
-        else TC_SPLIT_P(32);
-#undef TC_SPLIT_P
-    } else if (split && !persistent) {
-#define TC_SPLIT(BNV)                                                                  \
-    do {                                                                               \
-        if (!a_mn && !b_mn) launch_tc<BNV, false, false, true>(ma, mb, g, st);         \
-        else if (!a_mn && b_mn) launch_tc<BNV, false, true, true>(ma, mb, g, st);      \
-        else if (a_mn && !b_mn) launch_tc<BNV, true, false, true>(ma, mb, g, st);      \
-        else launch_tc<BNV, true, true, true>(ma, mb, g, st);                          \
-    } while (0)
-        if (bn == 128) TC_SPLIT(128);
-        else if (bn == 64) TC_SPLIT(64);
-        else TC_SPLIT(32);
-#undef TC_SPLIT
-    } else if (bn == 192) {
-        if (!a_mn && !b_mn) launch_tc<192, false, false>(ma, mb, g, st);
-        else if (!a_mn && b_mn) launch_tc<192, false, true>(ma, mb, g, st);
-        else if (a_mn && !b_mn) launch_tc<192, true, false>(ma, mb, g, st);
-        else launch_tc<192, true, true>(ma, mb, g, st);
-    } else if (bn == 128) TC_DISPATCH(128);
-    else if (bn == 64) TC_DISPATCH(64);
-    else TC_DISPATCH(32);
-#undef TC_DISPATCH
+    if (persistent) {
+        if (bn == 128) TC_PERSISTENT(128);
+        else if (bn == 64) TC_PERSISTENT(64);
+        else TC_PERSISTENT(32);
+    } else if (split) {
+        if (bn == 128) TC_LAYOUT(128, true);
+        else if (bn == 64) TC_LAYOUT(64, true);
+        else TC_LAYOUT(32, true);
+    } else if (bn == 192) TC_LAYOUT(192, false);
+    else if (bn == 128) TC_LAYOUT(128, false);
+    else if (bn == 64) TC_LAYOUT(64, false);
+    else TC_LAYOUT(32, false);
+#undef TC_PERSISTENT
+#undef TC_LAYOUT
     if (g.ksplit > 1) {
         long long total = (long long)M * N;
         int blocks = (int)((total + 255) / 256);
         if (blocks > 148 * 8) blocks = 148 * 8;
-        launch_pdl(tc_splitk_reduce_kernel, blocks, 256, 0, st, g);
+        launch_kernel(tc_splitk_reduce_kernel, blocks, 256, 0, st, g);
     }
     return check_launch("gb200_gemm_tc", g.ksplit > 1 ? 2 : 1);
+}
+}  // namespace gb200
+
+extern "C" int gb200_gemm_tc(int device, const float* A, int lda, int transA, const float* B, int ldb, int transB,
+                             float* C, int ldc, int M, int N, int K, float alpha, const float* bias, int act,
+                             float* Zout, int ldz, float drop_p, unsigned long long seed, const float* R, int ldr,
+                             float rscale, int accumulate, int ksplit, float* workspace, size_t workspace_bytes,
+                             int split, void* stream) {
+    return gemm_tc(device, A, lda, transA, B, ldb, transB, C, ldc, M, N, K, alpha, bias, act, Zout, ldz, drop_p, seed, R,
+                   ldr, rscale, accumulate, nullptr, 0, ACT_NONE, ksplit, workspace, workspace_bytes, split, stream);
 }
 
 extern "C" int gb200_gemm_tc_gated(int device, const float* A, int lda, int transA, const float* B, int ldb, int transB,
                                    float* C, int ldc, int M, int N, int K, float alpha, float drop_p,
                                    unsigned long long seed, float rscale, const float* gate, int ldg, int gate_act,
-                                   int ksplit, float* workspace, size_t workspace_bytes, void* stream) {
-    GemmGate& gg = next_gemm_gate();
-    gg.G = gate; gg.ldg = ldg; gg.act = gate_act;
-    const int rc = gb200_gemm_tc(device, A, lda, transA, B, ldb, transB, C, ldc, M, N, K, alpha, nullptr, ACT_NONE, nullptr,
-                                 0, drop_p, seed, nullptr, 0, rscale, 0, ksplit, workspace, workspace_bytes, stream);
-    gg.G = nullptr;
-    return rc;
+                                   int ksplit, float* workspace, size_t workspace_bytes, int split, void* stream) {
+    return gemm_tc(device, A, lda, transA, B, ldb, transB, C, ldc, M, N, K, alpha, nullptr, ACT_NONE, nullptr, 0, drop_p,
+                   seed, nullptr, 0, rscale, 0, gate, ldg, gate_act, ksplit, workspace, workspace_bytes, split, stream);
 }
 
 extern "C" size_t gb200_gemm_tc_wgrad_group_workspace_bytes(int n, const gb200_wgrad_problem* probs) {
@@ -1031,9 +935,8 @@ extern "C" int gb200_gemm_tc_wgrad_group(int device, int n, const gb200_wgrad_pr
         tiles += cdiv(q.M, TC_BM) * cdiv(q.N, 128);
     }
     // Grid size: two CTAs per SM over the whole GPU.  A smaller grid that would fit on the 28 SMs the fused encoder kernels
-    // leave free was measured (GB200_WGRAD_CTAS=56/112: 4.66/4.68 ms per C3 step against 4.61) -- filling the GPU wins.
-    static const int target = env_int("GB200_WGRAD_CTAS", 296);
-    int S = target / tiles;
+    // leave free was measured (56 / 112 CTAs: 4.66 / 4.68 ms per C3 step against 4.61) -- filling the GPU wins.
+    int S = 2 * 148 / tiles;
     if (S < 1) S = 1;
     if (S > 64) S = 64;
     size_t woff = 0;
@@ -1068,29 +971,4 @@ extern "C" int gb200_gemm_tc_wgrad_group(int device, int n, const gb200_wgrad_pr
     gemm_tc_group_kernel<128><<<cta, TC_THREADS, tc_smem_bytes<128>(), st>>>(G);
     tc_splitk_reduce_group_kernel<<<dim3(64, n), 256, 0, st>>>(G);
     return check_launch("gb200_gemm_tc_wgrad_group", 2);
-}
-
-/* y = x W^T + b with per-head LayerNorm statistics fused into the epilogue: columns [col_lo, col_hi) of the output
- * (two operand blocks of heads*dk columns each, e.g. K and V of the packed Q|K|V projection) are replaced by
- * (y - mean) * rstd per (row, head) and rstd is written to rstd_a / rstd_b (rows, heads).
- * libs/layers.py:837-839 + 846-851 in one kernel.  Requirements beyond gb200_gemm_tc: no activation / dropout /
- * residual / split-K, N % 4 == 0, dk % 4 == 0 with dk/4 a power of two <= 32, 32 % (dk/4) == 0, col_lo % dk == 0. */
-extern "C" int gb200_gemm_tc_headnorm(int device, const float* A, int lda, const float* W, int ldw, float* C, int ldc,
-                                      int M, int N, int K, const float* bias, int col_lo, int col_hi, int heads, int dk,
-                                      float eps, float* rstd_a, float* rstd_b, void* stream) {
-    const int lg = dk / 4;
-    GB_REQUIRE(dk % 4 == 0 && lg >= 1 && lg <= 32 && (lg & (lg - 1)) == 0, "gb200_gemm_tc_headnorm: unsupported d_k=%d", dk);
-    GB_REQUIRE(col_lo % dk == 0 && (col_hi - col_lo) % (heads * dk) == 0 && col_hi <= N && col_lo >= 0 &&
-                   (col_hi - col_lo) / (heads * dk) >= 1 && (col_hi - col_lo) / (heads * dk) <= 2,
-               "gb200_gemm_tc_headnorm: bad column range [%d, %d)", col_lo, col_hi);
-    GB_REQUIRE(rstd_a && ((col_hi - col_lo) / (heads * dk) == 1 || rstd_b), "gb200_gemm_tc_headnorm: null rstd");
-    GB_REQUIRE(N % 128 == 0 || N == 64 || N == 32, "gb200_gemm_tc_headnorm: N=%d must tile evenly", N);
-    GB_REQUIRE(N % 4 == 0 && ldc % 4 == 0 && ((uintptr_t)C % 16) == 0 && (!bias || ((uintptr_t)bias % 16) == 0),
-               "gb200_gemm_tc_headnorm: output must be float4-aligned");
-    g_hn.dk = dk; g_hn.lo = col_lo; g_hn.hi = col_hi; g_hn.heads = heads; g_hn.eps = eps;
-    g_hn.rstd[0] = rstd_a; g_hn.rstd[1] = rstd_b;
-    int rc = gb200_gemm_tc(device, A, lda, 0, W, ldw, 1, C, ldc, M, N, K, 1.f, bias, ACT_NONE, nullptr, 0, 0.f, 0, nullptr,
-                           0, 1.f, 0, 1, nullptr, 0, stream);
-    g_hn.dk = 0;
-    return rc;
 }

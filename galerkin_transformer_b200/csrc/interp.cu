@@ -309,26 +309,24 @@ static int launch_interp(bool backward, const float* in, float* out, int B, int 
     if (blocks > 148 * 32) blocks = 148 * 32;
     if (blocks < 1) blocks = 1;
     if (backward) {
-        static const int use_table = [] { const char* v = getenv("GB200_INTERP_TABLE"); return v ? atoi(v) : 1; }();
         const size_t smem = (size_t)Win * (IB_MAXR + 1) * sizeof(float);
-        if (use_table && max_candidates(a.sy, Hout) <= IB_MAXR && max_candidates(a.sx, Wout) <= IB_MAXR && smem <= 40 * 1024) {
-            if (vec) launch_pdl(interp_bwd_table_kernel<true>, (int)blocks, 256, smem, st, a);
-            else launch_pdl(interp_bwd_table_kernel<false>, (int)blocks, 256, smem, st, a);
+        if (max_candidates(a.sy, Hout) <= IB_MAXR && max_candidates(a.sx, Wout) <= IB_MAXR && smem <= 40 * 1024) {
+            if (vec) launch_kernel(interp_bwd_table_kernel<true>, (int)blocks, 256, smem, st, a);
+            else launch_kernel(interp_bwd_table_kernel<false>, (int)blocks, 256, smem, st, a);
         } else if (vec) {
-            launch_pdl(interp_bwd_kernel<true>, (int)blocks, 256, 0, st, a);
+            launch_kernel(interp_bwd_kernel<true>, (int)blocks, 256, 0, st, a);
         } else {
-            launch_pdl(interp_bwd_kernel<false>, (int)blocks, 256, 0, st, a);
+            launch_kernel(interp_bwd_kernel<false>, (int)blocks, 256, 0, st, a);
         }
     } else {
-        static const int use_table = [] { const char* v = getenv("GB200_INTERP_TABLE"); return v ? atoi(v) : 1; }();
         const size_t smem = (size_t)Wout * 3 * sizeof(float);
-        if (use_table && smem <= 40 * 1024) {
-            if (vec) launch_pdl(interp_fwd_table_kernel<true>, (int)blocks, 256, smem, st, a);
-            else launch_pdl(interp_fwd_table_kernel<false>, (int)blocks, 256, smem, st, a);
+        if (smem <= 40 * 1024) {
+            if (vec) launch_kernel(interp_fwd_table_kernel<true>, (int)blocks, 256, smem, st, a);
+            else launch_kernel(interp_fwd_table_kernel<false>, (int)blocks, 256, smem, st, a);
         } else if (vec) {
-            launch_pdl(interp_fwd_kernel<true>, (int)blocks, 256, 0, st, a);
+            launch_kernel(interp_fwd_kernel<true>, (int)blocks, 256, 0, st, a);
         } else {
-            launch_pdl(interp_fwd_kernel<false>, (int)blocks, 256, 0, st, a);
+            launch_kernel(interp_fwd_kernel<false>, (int)blocks, 256, 0, st, a);
         }
     }
     return check_launch(backward ? "gb200_interp_bilinear_bwd" : "gb200_interp_bilinear_fwd");

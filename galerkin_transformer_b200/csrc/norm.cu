@@ -91,7 +91,7 @@ extern "C" int gb200_layernorm_fwd(int device, const float* x, long long rows, i
     use_device(device);
     GB_REQUIRE(x && gamma && beta && y && mean && rstd && width >= 1, "gb200_layernorm_fwd: bad arguments");
     if (rows == 0) return GB200_OK;
-    launch_pdl(layernorm_fwd_kernel, ln_blocks(rows), LN_WARPS * 32, 0, as_stream(stream), x, rows, width, gamma, beta,
+    launch_kernel(layernorm_fwd_kernel, ln_blocks(rows), LN_WARPS * 32, 0, as_stream(stream), x, rows, width, gamma, beta,
                                                                                   eps, y, mean, rstd);
     return check_launch("gb200_layernorm_fwd");
 }
@@ -115,8 +115,8 @@ extern "C" int gb200_layernorm_bwd(int device, const float* dy, const float* x, 
     if (smem > 48 * 1024)
         cudaFuncSetAttribute(layernorm_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     cudaStream_t st = as_stream(stream);
-    launch_pdl(layernorm_bwd_kernel, nblocks, LN_WARPS * 32, smem, st, dy, x, mean, rstd, gamma, rows, width, dx, workspace);
-    launch_pdl(layernorm_bwd_reduce_kernel, dim3(cdiv(width, 32), 2), dim3(32, 32), 0, st, workspace, nblocks, width, dgamma,
+    launch_kernel(layernorm_bwd_kernel, nblocks, LN_WARPS * 32, smem, st, dy, x, mean, rstd, gamma, rows, width, dx, workspace);
+    launch_kernel(layernorm_bwd_reduce_kernel, dim3(cdiv(width, 32), 2), dim3(32, 32), 0, st, workspace, nblocks, width, dgamma,
                                                                                 dbeta, accumulate);
     return check_launch("gb200_layernorm_bwd", 2);
 }

@@ -1,10 +1,8 @@
 // Library-level plumbing: error strings, device selection, launch accounting.
 #include <atomic>
 #include <cstdarg>
-#include <cstdlib>
 
 #include "common.cuh"
-#include "gemm_epilogue.cuh"
 
 namespace gb200 {
 
@@ -14,19 +12,6 @@ static std::atomic<unsigned long long> g_launches{0};
 static const unsigned long long* g_rng_offset = nullptr;
 
 const unsigned long long* rng_offset_ptr() { return g_rng_offset; }
-
-GemmGate& next_gemm_gate() {
-    static thread_local GemmGate g = {nullptr, 0, 0};
-    return g;
-}
-
-bool pdl_enabled() {
-    static const bool on = [] {
-        const char* e = getenv("GB200_PDL");      // opt-in: measured SLOWER inside the captured step (DESIGN.md section 6)
-        return e && e[0] == '1';
-    }();
-    return on;
-}
 
 void set_error(const char* fmt, ...) {
     va_list ap;
@@ -55,7 +40,7 @@ int check_launch(const char* what, int nkernels) {
 
 }  // namespace gb200
 
-extern "C" int gb200_version(void) { return 101; }
+extern "C" int gb200_version(void) { return 102; }
 extern "C" int gb200_set_rng_offset_ptr(const unsigned long long* device_counter) {
     gb200::g_rng_offset = device_counter;
     return GB200_OK;
@@ -95,6 +80,6 @@ extern "C" int gb200_pack(int device, float* dst, const float* const* srcs, cons
     int by = (int)((biggest + 256 * 8 - 1) / (256 * 8));
     if (by < 1) by = 1;
     if (by > 32) by = 32;
-    launch_pdl(pack_kernel, dim3(n, by), 256, 0, as_stream(stream), a, dst);
+    launch_kernel(pack_kernel, dim3(n, by), 256, 0, as_stream(stream), a, dst);
     return check_launch("gb200_pack");
 }

@@ -407,13 +407,13 @@ __global__ void __launch_bounds__(128) ydft_row_kernel(const float* __restrict__
 // Channel-blocked forward transform: a thread owns 4 channels x YQ_KPT modes of one row and every YQ-th point of it, so each
 // twiddle word read from shared memory (a broadcast: 1 word per cycle, however wide the load) feeds 4 FMAs and each x
 // value (one float4 straight from global memory) feeds 2*YQ_KPT.  ncu showed the first version latency-bound (long-scoreboard
-// stalls at 23% occupancy): the point split is 8-way where the thread budget allows (twice the warps), the x loads are
-// double-buffered one batch ahead, and the twiddle table is filled with six independent loads per thread in flight.
+// stalls at 23% occupancy): the x loads are double-buffered one batch ahead, and the twiddle table is filled with six
+// independent loads per thread in flight.  The point split is 4-way (8-way, twice the warps, measured 35 against 21 us).
 // The YQ point groups are reduced through shared memory in fixed order.
+constexpr int YQ = 4;
 constexpr int YQ_KPT = 6;
 constexpr int YQ_UN = 6;
 
-template <int YQ>
 __global__ void __launch_bounds__(128) ydft_rowq_kernel(const float* __restrict__ x, long long R, int n, int P, int C, int m,
                                                         int CG, int KG, const float2* __restrict__ twY, float scale,
                                                         int hermitian, float2* __restrict__ out) {
@@ -740,10 +740,6 @@ __global__ void __launch_bounds__(512) yidft_row_kernel(
 }
 
 static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
-static int spectral_rows_enabled() {
-    static const int on = [] { const char* v = getenv("GB200_SPECTRAL_ROWS"); return v ? atoi(v) : 1; }();
-    return on;
-}
 
 }  // namespace gb200
 
@@ -783,7 +779,7 @@ extern "C" int gb200_spectral_ydft(int device, const float* x, long long R, int 
     do {                                                                                                       \
         if (smem > 48 * 1024)                                                                                  \
             cudaFuncSetAttribute(ydft_mma_kernel<NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-        launch_pdl(ydft_mma_kernel<NT>, grid, SM_WARPS * 32, smem, st, x, R, n, C, m, reinterpret_cast<const float2*>(twY), \
+        launch_kernel(ydft_mma_kernel<NT>, grid, SM_WARPS * 32, smem, st, x, R, n, C, m, reinterpret_cast<const float2*>(twY), \
                                                               scale, hermitian, reinterpret_cast<float2*>(out)); \
     } while (0)
         switch (C / 8) { case 1: YD(1); break; case 2: YD(2); break; case 3: YD(3); break; case 4: YD(4); break;
@@ -791,37 +787,26 @@ extern "C" int gb200_spectral_ydft(int device, const float* x, long long R, int 
 #undef YD
         return check_launch("gb200_spectral_ydft");
     }
-    if (spectral_rows_enabled() && nsplit == 1 && C % 4 == 0 && R >= 148 && R <= 0x7fffffffLL && aligned16(x) &&
-        aligned16(out)) {
+    if (nsplit == 1 && C % 4 == 0 && R >= 148 && R <= 0x7fffffffLL && aligned16(x) && aligned16(out)) {
         const int CG = C / 4, KG = cdiv(m, YQ_KPT), TPR = CG * KG;
         const int P = n | 1;                              // odd pitch: the KG mode groups of a warp fall in distinct banks
-        static const int yq_env = [] { const char* v = getenv("GB200_YDFT_YQ"); return v ? atoi(v) : 4; }();
-        const int YQ = (yq_env == 8 && TPR <= 16) ? 8 : 4;   // point split (8-way needs the row to fit the 128-thread CTA)
         const size_t smem = (size_t)(2 * KG * YQ_KPT * P + (YQ - 1) * (128 / YQ) * 2 * YQ_KPT * 4) * sizeof(float);
-        if (yq_env != 0 && TPR <= 32 && (TPR & (TPR - 1)) == 0 && smem <= 96 * 1024) {
+        if (TPR <= 32 && (TPR & (TPR - 1)) == 0 && smem <= 96 * 1024) {
             const int rows = (128 / YQ) / TPR;
-            if (YQ == 8) {
-                if (smem > 48 * 1024)
-                    cudaFuncSetAttribute(ydft_rowq_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-                launch_pdl(ydft_rowq_kernel<8>, dim3((unsigned)cdiv(R, rows)), 128, smem, st, x, R, n, P, C, m, CG, KG,
-                           reinterpret_cast<const float2*>(twY), scale, hermitian, reinterpret_cast<float2*>(out));
-            } else {
-                if (smem > 48 * 1024)
-                    cudaFuncSetAttribute(ydft_rowq_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-                launch_pdl(ydft_rowq_kernel<4>, dim3((unsigned)cdiv(R, rows)), 128, smem, st, x, R, n, P, C, m, CG, KG,
-                           reinterpret_cast<const float2*>(twY), scale, hermitian, reinterpret_cast<float2*>(out));
-            }
+            if (smem > 48 * 1024)
+                cudaFuncSetAttribute(ydft_rowq_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+            launch_kernel(ydft_rowq_kernel, dim3((unsigned)cdiv(R, rows)), 128, smem, st, x, R, n, P, C, m, CG, KG,
+                          reinterpret_cast<const float2*>(twY), scale, hermitian, reinterpret_cast<float2*>(out));
             return check_launch("gb200_spectral_ydft");
         }
     }
     {
         const int NP = (n + 3) / 4 * 4;
         const size_t smem = (size_t)(NP * C + 2 * m * NP) * sizeof(float);
-        if (spectral_rows_enabled() && nsplit == 1 && C % 4 == 0 && R >= 148 && R <= 0x7fffffffLL && smem <= 96 * 1024 &&
-            aligned16(x)) {
+        if (nsplit == 1 && C % 4 == 0 && R >= 148 && R <= 0x7fffffffLL && smem <= 96 * 1024 && aligned16(x)) {
             if (smem > 48 * 1024)
                 cudaFuncSetAttribute(ydft_row_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-            launch_pdl(ydft_row_kernel, dim3((unsigned)R), 128, smem, st, x, n, NP, C, m,
+            launch_kernel(ydft_row_kernel, dim3((unsigned)R), 128, smem, st, x, n, NP, C, m,
                        reinterpret_cast<const float2*>(twY), scale, hermitian, reinterpret_cast<float2*>(out));
             return check_launch("gb200_spectral_ydft");
         }
@@ -831,14 +816,14 @@ extern "C" int gb200_spectral_ydft(int device, const float* x, long long R, int 
     nsplit = cdiv(n, ychunk);
     dim3 grid(cdiv(RC, 128), nsplit, cdiv(m, KYG));
     GB_REQUIRE(grid.y <= 65535 && grid.z <= 65535, "gb200_spectral_ydft: grid too large");
-    launch_pdl(ydft_kernel, grid, 128, 0, st, x, RC, C, n, m, reinterpret_cast<const float2*>(twY), scale, hermitian,
+    launch_kernel(ydft_kernel, grid, 128, 0, st, x, RC, C, n, m, reinterpret_cast<const float2*>(twY), scale, hermitian,
                                       nsplit, ychunk, reinterpret_cast<float2*>(out),
                                       reinterpret_cast<float2*>(workspace));
     if (nsplit > 1) {
         long long total = R * m * C;
         int blocks = (int)((total + 255) / 256);
         if (blocks > 148 * 8) blocks = 148 * 8;
-        launch_pdl(ydft_reduce_kernel, blocks, 256, 0, st, reinterpret_cast<const float2*>(workspace), nsplit, total, C,
+        launch_kernel(ydft_reduce_kernel, blocks, 256, 0, st, reinterpret_cast<const float2*>(workspace), nsplit, total, C,
                                                    m, n, scale, hermitian, reinterpret_cast<float2*>(out));
     }
     return check_launch("gb200_spectral_ydft", nsplit > 1 ? 2 : 1);
@@ -850,11 +835,11 @@ extern "C" int gb200_spectral_xdft(int device, const float* T1, int B, int n, in
     GB_REQUIRE(T1 && twX && out && B >= 1 && n >= 1 && m >= 1 && C >= 1, "gb200_spectral_xdft: bad arguments");
     GB_REQUIRE(2 * m <= n, "gb200_spectral_xdft: 2*modes=%d exceeds n=%d (mode blocks would overlap)", 2 * m, n);
     cudaStream_t st = as_stream(stream);
-    if (spectral_rows_enabled() && B <= 65535 && m <= 65535) {
+    if (B <= 65535 && m <= 65535) {
         if (!inverse) {
             const size_t smem = (size_t)XD_RG * n * sizeof(float2);
             if (smem <= 36 * 1024) {          // + 10.5 KB of static reduction buffer: stays under the 48 KB default limit
-                launch_pdl(xdft_rows_kernel, dim3(cdiv(2 * m, XD_RG), m, B), 32 * XD_XQ, smem, st,
+                launch_kernel(xdft_rows_kernel, dim3(cdiv(2 * m, XD_RG), m, B), 32 * XD_XQ, smem, st,
                            reinterpret_cast<const float2*>(T1), n, m, C, reinterpret_cast<const float2*>(twX), scale,
                            reinterpret_cast<float2*>(out));
                 return check_launch("gb200_spectral_xdft");
@@ -862,7 +847,7 @@ extern "C" int gb200_spectral_xdft(int device, const float* T1, int B, int n, in
         } else {
             const size_t smem = (size_t)2 * m * (32 + XI_XC) * sizeof(float2);
             if (smem <= 48 * 1024) {
-                launch_pdl(xidft_rows_kernel, dim3(cdiv(n, XI_XC), m, B), 128, smem, st,
+                launch_kernel(xidft_rows_kernel, dim3(cdiv(n, XI_XC), m, B), 128, smem, st,
                            reinterpret_cast<const float2*>(T1), n, m, C, reinterpret_cast<const float2*>(twX), scale,
                            reinterpret_cast<float2*>(out));
                 return check_launch("gb200_spectral_xdft");
@@ -871,12 +856,12 @@ extern "C" int gb200_spectral_xdft(int device, const float* T1, int B, int n, in
     }
     if (!inverse) {
         long long total = (long long)B * 2 * m * m * C;
-        launch_pdl(xdft_kernel, cdiv(total, 128), 128, 0, st, reinterpret_cast<const float2*>(T1), B, n, m, C,
+        launch_kernel(xdft_kernel, cdiv(total, 128), 128, 0, st, reinterpret_cast<const float2*>(T1), B, n, m, C,
                                                       reinterpret_cast<const float2*>(twX), scale,
                                                       reinterpret_cast<float2*>(out));
     } else {
         long long total = (long long)B * n * m * C;
-        launch_pdl(xidft_kernel, cdiv(total, 256), 256, 0, st, reinterpret_cast<const float2*>(T1), B, n, m, C,
+        launch_kernel(xidft_kernel, cdiv(total, 256), 256, 0, st, reinterpret_cast<const float2*>(T1), B, n, m, C,
                                                        reinterpret_cast<const float2*>(twX), scale,
                                                        reinterpret_cast<float2*>(out));
     }
@@ -892,7 +877,7 @@ extern "C" int gb200_spectral_mix_fwd(int device, const float* Xf, const float* 
     int th = mix_threads(M2);
     dim3 grid(cdiv(M2, th), Co, halves * cdiv(B, MIXB));
     GB_REQUIRE(grid.y <= 65535 && grid.z <= 65535, "gb200_spectral_mix_fwd: grid too large");
-    launch_pdl(mix_fwd_kernel, grid, th, 0, as_stream(stream), reinterpret_cast<const float2*>(Xf),
+    launch_kernel(mix_fwd_kernel, grid, th, 0, as_stream(stream), reinterpret_cast<const float2*>(Xf),
                                                        reinterpret_cast<const float2*>(W0),
                                                        reinterpret_cast<const float2*>(W1), B, halves, M2, Ci, Co,
                                                        reinterpret_cast<float2*>(Of));
@@ -908,7 +893,7 @@ extern "C" int gb200_spectral_mix_bwd(int device, const float* Xf, const float* 
     cudaStream_t st = as_stream(stream);
     if (dX) {
         dim3 grid(cdiv(M2, th), Ci, halves * cdiv(B, MIXB));
-        launch_pdl(mix_bwd_x_kernel, grid, th, 0, st, reinterpret_cast<const float2*>(dO),
+        launch_kernel(mix_bwd_x_kernel, grid, th, 0, st, reinterpret_cast<const float2*>(dO),
                                               reinterpret_cast<const float2*>(W0),
                                               reinterpret_cast<const float2*>(W1), B, halves, M2, Ci, Co,
                                               reinterpret_cast<float2*>(dX));
@@ -916,7 +901,7 @@ extern "C" int gb200_spectral_mix_bwd(int device, const float* Xf, const float* 
     if (dW0) {
         GB_REQUIRE(halves == 1 || dW1, "gb200_spectral_mix_bwd: dW1 is null");
         dim3 grid(cdiv(M2, th), Co, halves);
-        launch_pdl(mix_bwd_w_kernel, grid, th, 0, st, reinterpret_cast<const float2*>(Xf),
+        launch_kernel(mix_bwd_w_kernel, grid, th, 0, st, reinterpret_cast<const float2*>(Xf),
                                               reinterpret_cast<const float2*>(dO), B, halves, M2, Ci, Co,
                                               reinterpret_cast<float2*>(dW0), reinterpret_cast<float2*>(dW1),
                                               accumulate_dw);
@@ -950,7 +935,7 @@ extern "C" int gb200_spectral_yidft_epilogue(int device, const float* Z, long lo
     do {                                                                                                         \
         if (smem2 > 48 * 1024)                                                                                   \
             cudaFuncSetAttribute(yidft_mma_kernel<NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2); \
-        launch_pdl(yidft_mma_kernel<NT>, grid, SM_WARPS * 32, smem2, st2, \
+        launch_kernel(yidft_mma_kernel<NT>, grid, SM_WARPS * 32, smem2, st2, \
             reinterpret_cast<const float2*>(Z), R, n, m, Co, reinterpret_cast<const float2*>(twY), scale, hermitian, \
             x2, Ci, Wm, bias, act, y, zout, tiles_per_warp, chunks);                                             \
     } while (0)
@@ -960,7 +945,7 @@ extern "C" int gb200_spectral_yidft_epilogue(int device, const float* Z, long lo
             return check_launch("gb200_spectral_yidft_epilogue");
         }
     }
-    if (spectral_rows_enabled() && Co % 8 == 0 && Co <= 128 && Ci % 4 == 0 && R >= 148 && aligned16(x2) && aligned16(Wm) &&
+    if (Co % 8 == 0 && Co <= 128 && Ci % 4 == 0 && R >= 148 && aligned16(x2) && aligned16(Wm) &&
         aligned16(y) && (!zout || aligned16(zout)) && (!bias || aligned16(bias))) {
         const int OG = Co / 4;
         const int pad12 = cdiv(n, 48) * 48, pad16 = cdiv(n, 64) * 64;
@@ -976,12 +961,12 @@ extern "C" int gb200_spectral_yidft_epilogue(int device, const float* Z, long lo
             if (YG == 12) {
                 if (smr > 48 * 1024)
                     cudaFuncSetAttribute(yidft_row_kernel<12>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smr);
-                launch_pdl(yidft_row_kernel<12>, gridr, threads, smr, str, reinterpret_cast<const float2*>(Z), n, m, Co,
+                launch_kernel(yidft_row_kernel<12>, gridr, threads, smr, str, reinterpret_cast<const float2*>(Z), n, m, Co,
                            reinterpret_cast<const float2*>(twY), scale, hermitian, x2, Ci, Wm, bias, act, y, zout, tpc);
             } else {
                 if (smr > 48 * 1024)
                     cudaFuncSetAttribute(yidft_row_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smr);
-                launch_pdl(yidft_row_kernel<16>, gridr, threads, smr, str, reinterpret_cast<const float2*>(Z), n, m, Co,
+                launch_kernel(yidft_row_kernel<16>, gridr, threads, smr, str, reinterpret_cast<const float2*>(Z), n, m, Co,
                            reinterpret_cast<const float2*>(twY), scale, hermitian, x2, Ci, Wm, bias, act, y, zout, tpc);
             }
             return check_launch("gb200_spectral_yidft_epilogue");
@@ -996,7 +981,7 @@ extern "C" int gb200_spectral_yidft_epilogue(int device, const float* Z, long lo
     int tiles_per_cta = ntiles;
     while (tiles_per_cta > 1 && R * cdiv(ntiles, tiles_per_cta) < 4 * 148) tiles_per_cta = (tiles_per_cta + 1) / 2;
     dim3 grid((unsigned)R, cdiv(ntiles, tiles_per_cta));
-    launch_pdl(yidft_epi_kernel, grid, 256, smem, as_stream(stream), reinterpret_cast<const float2*>(Z), n, m, Co,
+    launch_kernel(yidft_epi_kernel, grid, 256, smem, as_stream(stream), reinterpret_cast<const float2*>(Z), n, m, Co,
                                                             reinterpret_cast<const float2*>(twY), scale, hermitian,
                                                             x2, Ci, Wm, bias, act, y, zout, tiles_per_cta);
     return check_launch("gb200_spectral_yidft_epilogue");

@@ -285,8 +285,8 @@ extern "C" int gb200_weighted_l2_loss2d(int device, const float* preds, const fl
     a.chunks = loss_chunks(B, n); a.ws = workspace; a.out = out4; a.dl = dloss; a.dr = dreg;
     cudaStream_t st = as_stream(stream);
     dim3 grid(a.chunks, B);
-    launch_pdl(loss_partial_kernel, grid, LOSS_THREADS, 0, st, a);
-    launch_pdl(loss_grad_kernel, grid, LOSS_THREADS, 0, st, a);
+    launch_kernel(loss_partial_kernel, grid, LOSS_THREADS, 0, st, a);
+    launch_kernel(loss_grad_kernel, grid, LOSS_THREADS, 0, st, a);
     return check_launch("gb200_weighted_l2_loss2d", 2);
 }
 
@@ -308,12 +308,12 @@ extern "C" int gb200_adam_clip_step(int device, float* param, const float* grad,
     GB_REQUIRE(workspace_bytes >= gb200_adam_clip_step_workspace_bytes(n), "gb200_adam_clip_step: workspace too small");
     cudaStream_t st = as_stream(stream);
     const int parts = adam_parts(n);
-    launch_pdl(sumsq_partial_kernel, parts, ADAM_THREADS, 0, st, grad, n, workspace);
+    launch_kernel(sumsq_partial_kernel, parts, ADAM_THREADS, 0, st, grad, n, workspace);
     AdamArgs a;
     a.p = param; a.m = exp_avg; a.v = exp_avg_sq; a.g = grad; a.n = n; a.hyper = hyper; a.beta2 = beta2; a.eps = eps;
     a.weight_decay = weight_decay; a.max_norm = max_norm; a.parts = workspace; a.nparts = parts; a.norm_out = grad_norm_out;
     long long blocks = (n + ADAM_THREADS * 4 - 1) / (ADAM_THREADS * 4);
     if (blocks > 148 * 8) blocks = 148 * 8;
-    launch_pdl(adam_kernel, (int)blocks, ADAM_THREADS, 0, st, a);
+    launch_kernel(adam_kernel, (int)blocks, ADAM_THREADS, 0, st, a);
     return check_launch("gb200_adam_clip_step", 2);
 }

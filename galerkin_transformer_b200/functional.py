@@ -28,10 +28,6 @@ ACT = {"none": 0, None: 0, "identity": 0, "relu": 1, "silu": 2}
 #   "tf32" every GEMM single-pass TF32 on tcgen05 (fastest unfused path; ~1e-2 gradient error through 10 layers)
 #   "fp32" exact-fp32 SIMT FMAs everywhere (the precise mode used by the tight parity tests).
 _PRECISION = "x3"
-# fold the K,V per-head LayerNorm statistics into the Q|K|V projection's tcgen05 epilogue (A/B switch)
-# -- measured 0.17 ms/step SLOWER at C3 than the separate coalesced headnorm kernel (the epilogue runs on 4 warps per
-# CTA, the stand-alone kernel on the whole GPU), so it is opt-in: GB200_FUSE_HEADNORM=1
-_FUSE_HEADNORM = __import__("os").environ.get("GB200_FUSE_HEADNORM", "0") == "1"
 
 
 def set_precision(mode):
@@ -50,7 +46,7 @@ def get_precision():
 
 torch.backends.cudnn.allow_tf32 = _PRECISION == "tf32"
 
-_SPLIT_MIN_FLOPS = float(os.environ.get("GB200_SPLIT_MIN_GFLOP", "0.5")) * 1e9   # measured: C5's 0.15 GFLOP GEMMs lose, C3's 1.3 win
+_SPLIT_MIN_FLOPS = 0.5e9   # measured: C5's 0.15 GFLOP GEMMs lose, C3's 1.3 win
 _seed_lock = threading.Lock()
 _seed_counter = 0
 
@@ -226,7 +222,7 @@ def aux_stream(device):
 
 _pending_joins = []
 _join_queued = False
-_DEFER_WGRAD_JOIN = os.environ.get("GB200_DEFER_WGRAD_JOIN", "1") != "0"
+_DEFER_WGRAD_JOIN = True      # graphs.GraphedStep clears it for concurrent micro-batch chains
 
 
 def _join_pending():
@@ -271,7 +267,7 @@ def _finish_fork(fork, params, keepalive):
     """End of a backward node whose parameter gradients were launched on side streams: normally the launching stream joins
     them only when the whole backward pass has been enqueued (they then overlap every later node instead of the rest of
     this one).  That needs autograd to ADOPT the gradient tensors (`p.grad is None`: no accumulation kernel on the
-    launching stream before the side stream has written them) -- otherwise, or with GB200_DEFER_WGRAD_JOIN=0, join now.
+    launching stream before the side stream has written them) -- otherwise, or with _DEFER_WGRAD_JOIN cleared, join now.
     `keepalive`: the tensors the side work reads (not its outputs: a second reference would make autograd copy them)."""
     if _single_use(params) and _DEFER_WGRAD_JOIN:
         fork.join_at_end_of_backward(keepalive)
@@ -293,21 +289,22 @@ def gemm(A, B, C, M, N, K, *, lda, ldb, ldc, transA=False, transB=False, alpha=1
     nbytes = 4.0 * (M * K + K * N + M * N * (1 + (residual is not None) + (zout is not None) + (gate is not None)))
     lay = ("t" if transA else "n") + ("t" if transB else "n")
     use_tc = _PRECISION in ("tf32", "x3") and lib.gb200_gemm_tc_supported(pa, lda, pb, ldb, M, N, K)
-    if use_tc and _PRECISION == "x3" and not wgrad:
-        if 2.0 * M * N * K < _SPLIT_MIN_FLOPS:  # small problems: the exact SIMT kernel has the shorter fixed latency
-            use_tc = False
-        else:
-            lib.gb200_gemm_tc_split_next(1)    # forward / input-gradient GEMM outside the fused kernels: 3xTF32
+    # forward / input-gradient GEMM outside the fused kernels in 'x3' mode: 3xTF32
+    split = use_tc and _PRECISION == "x3" and not wgrad
+    if split and 2.0 * M * N * K < _SPLIT_MIN_FLOPS:   # small problems: the exact SIMT kernel has the shorter fixed latency
+        use_tc = split = False
     if gate is not None:
         assert bias is None and act == 0 and zout is None and residual is None and not accumulate
         if ksplit is None:
             ksplit = lib.gb200_gemm_tc_suggest_ksplit(M, N, K) if use_tc else lib.gb200_gemm_suggest_ksplit(M, N, K, 1)
         ws_bytes = ksplit * M * N * 4 if ksplit > 1 else 0
         ws = workspace(ws_bytes, C)
-        fn = lib.gb200_gemm_tc_gated if use_tc else lib.gb200_gemm_gated
-        _launch(("gemm_tc_" if use_tc else "gemm_simt_") + lay, 2.0 * M * N * K, nbytes, fn, _dev(C), pa, lda, int(transA),
-                pb, ldb, int(transB), ptr(C) + 4 * c_off, ldc, M, N, K, alpha, drop_p, seed, rscale, ptr(gate), ldg,
-                gate_act, ksplit, ptr(ws), ws_bytes, stream_of(C))
+        args = (_dev(C), pa, lda, int(transA), pb, ldb, int(transB), ptr(C) + 4 * c_off, ldc, M, N, K, alpha, drop_p, seed,
+                rscale, ptr(gate), ldg, gate_act, ksplit, ptr(ws), ws_bytes)
+        if use_tc:
+            _launch("gemm_tc_" + lay, 2.0 * M * N * K, nbytes, lib.gb200_gemm_tc_gated, *args, int(split), stream_of(C))
+        else:
+            _launch("gemm_simt_" + lay, 2.0 * M * N * K, nbytes, lib.gb200_gemm_gated, *args, stream_of(C))
         return
     if use_tc:
         if ksplit is None:
@@ -316,7 +313,7 @@ def gemm(A, B, C, M, N, K, *, lda, ldb, ldc, transA=False, transB=False, alpha=1
         ws = workspace(ws_bytes, C)
         _launch("gemm_tc_" + lay, 2.0 * M * N * K, nbytes, lib.gb200_gemm_tc, _dev(C), pa, lda, int(transA), pb,
                 ldb, int(transB), ptr(C) + 4 * c_off, ldc, M, N, K, alpha, ptr(bias), act, ptr(zout), ldz, drop_p,
-                seed, ptr(residual), ldr, rscale, int(accumulate), ksplit, ptr(ws), ws_bytes, stream_of(C))
+                seed, ptr(residual), ldr, rscale, int(accumulate), ksplit, ptr(ws), ws_bytes, int(split), stream_of(C))
         return
     if ksplit is None:
         ksplit = lib.gb200_gemm_suggest_ksplit(M, N, K, 1)
@@ -327,15 +324,10 @@ def gemm(A, B, C, M, N, K, *, lda, ldb, ldc, transA=False, transB=False, alpha=1
             drop_p, seed, ptr(residual), ldr, rscale, int(accumulate), ksplit, ptr(ws), ws_bytes, stream_of(C))
 
 
-_DIAG_SKIP_WGRAD = os.environ.get("GB200_DIAG_SKIP_WGRAD", "0") == "1"
-
-
 def wgrad_group(problems, T):
     """[(G (T, M) view, M, ldg, X (T, N), N, dW (M, N)), ...] (at most 6): dW = G^T X for each, one tcgen05 TF32 split-K launch
     and one deterministic reduction for the whole group (gb200_gemm_tc_wgrad_group)."""
     lib = _lib.load()
-    if _DIAG_SKIP_WGRAD:          # timing diagnostics only (tools/): the gradients are then garbage
-        return
     n = len(problems)
     arr = (_lib.WgradProblem * n)()
     flops = nbytes = 0.0
@@ -840,24 +832,15 @@ class _LinearAttentionFn(torch.autograd.Function):
         qkv = torch.empty((T, 3 * dm), dtype=torch.float32, device=query.device)
         xs = [t.reshape(T, dm) for t in (query, key, value)]
         blocks = {"kv": (1, 2), "qk": (1, 0), None: ()}[norm_on]
-        lgq = dk // 4
-        fuse_norm = (_FUSE_HEADNORM and self_attn and _PRECISION == "tf32" and norm_on == "kv" and dk % 4 == 0 and 1 <= lgq <= 32
-                     and (lgq & (lgq - 1)) == 0 and (3 * dm) % 128 == 0 and dm % 4 == 0
-                     and lib.gb200_gemm_tc_supported(ptr(xs[0]), dm, ptr(wqkv), dm, T, 3 * dm, dm))
         rstd = []
-        if fuse_norm:      # one tcgen05 GEMM: Q|K|V projection with the K,V per-head LayerNorm statistics in its epilogue
-            rstd = [torch.empty((T, H), dtype=torch.float32, device=query.device) for _ in blocks]
-            _launch("gemm_tc_nt", 2.0 * T * 3 * dm * dm, 4.0 * (T * dm + 3 * dm * dm + T * 3 * dm),
-                    lib.gb200_gemm_tc_headnorm, dev, ptr(xs[0]), dm, ptr(wqkv), dm, ptr(qkv), 3 * dm, T, 3 * dm, dm,
-                    ptr(bqkv), dm, 3 * dm, H, dk, eps, ptr(rstd[0]), ptr(rstd[1]), st)
-        elif self_attn:      # one GEMM, N = 3*d_model
+        if self_attn:      # one GEMM, N = 3*d_model
             gemm(xs[0], wqkv, qkv, T, 3 * dm, dm, lda=dm, ldb=dm, ldc=3 * dm, transB=True, bias=bqkv)
         else:
             for i in range(3):
                 gemm(xs[i], wqkv, qkv, T, dm, dm, lda=dm, ldb=dm, ldc=3 * dm, transB=True,
                      bias=bqkv[i * dm:(i + 1) * dm], b_off=i * dm * dm, c_off=i * dm)
         # which blocks are normalised: galerkin -> (K, V), fourier -> (Q, K)
-        if blocks and not fuse_norm:      # both normalised operand blocks in ONE launch
+        if blocks:      # both normalised operand blocks in ONE launch
             rstd = [torch.empty((T, H), dtype=torch.float32, device=query.device) for _ in blocks]
             _launch("headnorm_fwd", 16.0 * T * dm, 16.0 * T * dm, lib.gb200_headnorm_fwd, dev, ptr(qkv), 3 * dm,
                     blocks[0] * dm, blocks[1] * dm, T, H, dk, eps, ptr(rstd[0]), ptr(rstd[1]), st)
@@ -1038,11 +1021,10 @@ def linear_attention(query, key, value, pos, flat, has_norm, keep_mask, *, n_hea
 # ------------------------------------------------------------------------------------------
 # Fused encoder layer (csrc/encoder_fwd.cu): three tcgen05 kernels per layer forward
 # ------------------------------------------------------------------------------------------
-_FUSED_BACKWARD = os.environ.get("GB200_FUSED_BACKWARD", "1") != "0"     # A/B switch: 0 = per-operator backward
 # The launching stream joins the weight-gradient side stream only when the whole backward pass is enqueued (autograd engine
 # callback), so the grouped weight-gradient GEMM of layer l overlaps the input-gradient chain of layers l-1, l-2, ...
-# Measured at C3 with the grouped launch: 4.82 -> 4.67 ms/step.  GB200_DEFER_WGRAD_JOIN=0 joins per layer (graphs.GraphedStep does
-# that itself for concurrent micro-batch chains, whose per-chain streams are joined before the backward pass ends).
+# Measured at C3 with the grouped launch: 4.82 -> 4.67 ms/step.  Joining per layer instead is what graphs.GraphedStep
+# selects for concurrent micro-batch chains, whose per-chain streams are joined before the backward pass ends
 # (_DEFER_WGRAD_JOIN is defined next to _Fork)
 
 
@@ -1147,7 +1129,7 @@ class _EncoderLayerFn(torch.autograd.Function):
         if dy is None:
             dy = torch.zeros_like(x)
         dy2 = dy.reshape(T, dm).contiguous()
-        if dA_ext is None and _FUSED_BACKWARD:
+        if dA_ext is None:       # the per-operator backward below also differentiates through the returned attention matrix
             return _EncoderLayerFn._backward_fused(ctx, dy2, x, pos, keep_mask, qkv, A, heads, x1, hid, packed, rstd, params)
         # FeedForward + shortcut
         c = _Ctx((x1, w1, w2, hid, None), (ACT["relu"], pf, seedf, p2, seed2, 1.0, True, True, True), (True,) * 12)

@@ -72,20 +72,19 @@ int gb200_gemm(int device, const float* A, int lda, int transA, const float* B, 
  * aligned operands with lda, ldb multiples of 4 and N, K >= 8 (gb200_gemm_tc_supported); otherwise call
  * gb200_gemm.  Relative error ~4e-4 per contraction (TF32), see DESIGN.md. */
 int gb200_gemm_tc_supported(const float* A, int lda, const float* B, int ldb, int M, int N, int K);
-/* One-shot: the next gb200_gemm_tc / gb200_gemm_tc_gated call of this thread runs in split ("3xTF32") arithmetic -- each
- * product is hi.hi + hi.lo + lo.hi of the two-term TF32 split of its fp32 operands (~2^-22 relative error): the tensor-core
- * path of the forward / input-gradient GEMMs in 'x3' precision mode where no fused kernel applies. */
-int gb200_gemm_tc_split_next(int on);
 int gb200_gemm_tc_suggest_ksplit(int M, int N, int K);
 /* Diagnostics: when `device_buffer` is non-null every CTA of subsequent gb200_gemm_tc launches writes eight
  * %globaltimer stamps (entry, setup done, first/last tile landed, last tile rounded, accumulator complete,
  * TMEM drained, stores issued) to device_buffer[8 * linear_cta + slot].  Null (default) disables it. */
 int gb200_gemm_tc_set_trace(unsigned long long* device_buffer);
+/* split != 0 runs the GEMM in split ("3xTF32") arithmetic -- each product is hi.hi + hi.lo + lo.hi of the two-term TF32
+ * split of its fp32 operands (~2^-22 relative error): the tensor-core path of the forward / input-gradient GEMMs in 'x3'
+ * precision mode where no fused kernel applies.  Same for gb200_gemm_tc_gated. */
 int gb200_gemm_tc(int device, const float* A, int lda, int transA, const float* B, int ldb, int transB,
                   float* C, int ldc, int M, int N, int K, float alpha, const float* bias, int act,
                   float* Zout, int ldz, float drop_p, unsigned long long seed, const float* R, int ldr,
                   float rscale, int accumulate, int ksplit, float* workspace, size_t workspace_bytes,
-                  void* stream);
+                  int split, void* stream);
 
 /* Grouped weight gradients: dW_i (M_i, N_i) = G_i^T X_i, i < n <= 6, each a contraction over all T_i rows (tokens), as ONE
  * tcgen05 TF32 split-K grid plus ONE fixed-order reduction -- the four weight gradients of an encoder layer
@@ -109,19 +108,11 @@ int gb200_gemm_tc_wgrad_group(int device, int n, const gb200_wgrad_problem* prob
 int gb200_gemm_tc_gated(int device, const float* A, int lda, int transA, const float* B, int ldb, int transB,
                         float* C, int ldc, int M, int N, int K, float alpha, float drop_p, unsigned long long seed,
                         float rscale, const float* gate, int ldg, int gate_act, int ksplit, float* workspace,
-                        size_t workspace_bytes, void* stream);
+                        size_t workspace_bytes, int split, void* stream);
 int gb200_gemm_gated(int device, const float* A, int lda, int transA, const float* B, int ldb, int transB,
                      float* C, int ldc, int M, int N, int K, float alpha, float drop_p, unsigned long long seed,
                      float rscale, const float* gate, int ldg, int gate_act, int ksplit, float* workspace,
                      size_t workspace_bytes, void* stream);
-
-/* C = A W^T + bias on the tensor cores with per-head LayerNorm statistics fused into the epilogue: output columns
- * [col_lo, col_hi) -- one or two operand blocks of heads*dk columns, e.g. K and V of the packed Q|K|V projection --
- * are replaced by (y - mean) * rstd per (row, head); rstd goes to rstd_a / rstd_b (rows, heads).
- * libs/layers.py:837-839 + 846-851 in one kernel (the affine part is applied on load by the attention kernels). */
-int gb200_gemm_tc_headnorm(int device, const float* A, int lda, const float* W, int ldw, float* C, int ldc, int M, int N,
-                           int K, const float* bias, int col_lo, int col_hi, int heads, int dk, float eps,
-                           float* rstd_a, float* rstd_b, void* stream);
 
 /* out[n] (+)= scale * sum_m X[m,n]            (bias gradients) */
 size_t gb200_colsum_workspace_bytes(long long M, int N);
